@@ -20,6 +20,7 @@ by the closed-form moment kernel, pdmpflux_moments_reduce and (N > 1) pdmpflux_m
   strong_scaling  BASELINE config 5 (FECMC / Boomerang d = 1000): 65536 chains in total sharded over the N ranks
   cpu_baseline  the C restatement of the reference (oracle/, OpenMP, one chain per thread) on the host cores
 `--impl reference` times that CPU restatement alone (Julia, hence the reference itself, is not installed).
+`--dump-outputs DIR` writes the last timed step's history and moment sums (a seeded sample of chains, < 64 MB) as .npy.
 """
 import argparse
 import json
@@ -268,6 +269,27 @@ def init_states(torch, dev, name, nch):
     return x0, v0
 
 
+DUMP_BYTES = 60 * 10 ** 6   # array data of --dump-outputs; with the .npy headers the directory stays below 64 MB
+
+
+def dump_outputs(out_dir, bufs, m1, m2, T, sums, seed=0):
+    """Write what the last timed step handed back as out_dir/<name>.npy in float64: the 4 x d moment sums whole, and
+    for a fixed, seeded sample of chains (as many as fit in DUMP_BYTES, in chain order) every history column and the
+    chain's moments.  Same arguments give the same inputs, so two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    per_chain = dict(bufs, chain_m1=m1, chain_m2=m2, chain_T=T)
+    nch = T.shape[0]
+    chain_bytes = sum(a[0].numel() for a in per_chain.values()) * 8
+    k = min(nch, max(1, (DUMP_BYTES - sums.numel() * 8) // chain_bytes))
+    idx = np.sort(np.random.default_rng(seed).choice(nch, size=k, replace=False))
+    sel = torch.from_numpy(idx).to(T.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "moment_sums.npy"), sums.cpu().numpy())
+    for name, a in per_chain.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.index_select(0, sel).cpu().numpy().astype(np.float64))
+
+
 C4_ROWS, C4_GRID = 100000, 10
 
 
@@ -330,7 +352,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -436,6 +463,8 @@ def main():
         pass
     hbm_peak = float(peaks.get("hbm_gbs", 6650.0))
     peak_src = "MEASURED_PEAKS.json hbm_gbs (measured copy)" if peaks else "fallback 6.65 TB/s"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bufs, m1, m2, Tl, sums)
     chains.close()
     del bufs, view
     torch.cuda.empty_cache()
