@@ -361,31 +361,50 @@ __global__ void __launch_bounds__(256) speedup_scalars_kernel(int d, int64_t n_r
 }
 
 // Closed-form time integrals of x_i and x_i^2 along each chain's piecewise flow (feeds moments / ESS).
-__global__ void __launch_bounds__(256) moments_kernel(int flow_kind, int d, int64_t n_sk, int64_t n_chains,
-                                                      int64_t col_begin, const double* __restrict__ X,
-                                                      const double* __restrict__ V, const double* __restrict__ T,
-                                                      double* __restrict__ m1, double* __restrict__ m2,
-                                                      double* __restrict__ Tlen) {
+// One thread per (chain, coordinate) sums its segments in event order.  The pass streams X and V once (3.3 GB at
+// the bench shape), so what bounds it is the bytes in flight: the event loop is unrolled by kMomU and the loads of a
+// whole batch are issued before its arithmetic, and the linear flow keeps 6 blocks per SM (40 registers) so the
+// 800 blocks of the bench shape (4096 chains x d = 50) fit in one wave instead of leaving a 60-block tail (the
+// rotation flow's sincos needs more registers: 4 blocks).
+constexpr int kMomU = 4;
+template <int FLOW>
+__device__ __forceinline__ void moment_segment(double tau, double x, double v, double& s1, double& s2) {
+    if constexpr (FLOW == 1) {
+        double s, co;
+        sincos(tau, &s, &co);
+        const double s2t = 2.0 * s * co;  // sin(2 tau)
+        s1 += x * s + v * (1.0 - co);
+        s2 += x * x * (0.5 * tau + 0.25 * s2t) + v * v * (0.5 * tau - 0.25 * s2t) + x * v * s * s;
+    } else {
+        s1 += tau * (x + 0.5 * v * tau);
+        s2 += tau * (x * x + tau * (x * v + v * v * tau * (1.0 / 3.0)));
+    }
+}
+template <int FLOW>
+__global__ void __launch_bounds__(256, FLOW == 1 ? 4 : 6) moments_kernel(int d, int64_t n_sk, int64_t n_chains, int64_t col_begin,
+                                                         const double* __restrict__ X, const double* __restrict__ V,
+                                                         const double* __restrict__ T, double* __restrict__ m1,
+                                                         double* __restrict__ m2, double* __restrict__ Tlen) {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_chains * d) return;
     const int64_t c = e / d;
     const int a = (int)(e - c * d);
     const double* t = T + c * n_sk;
+    const double* tp = t + col_begin;
+    const double* xp = X + (c * n_sk + col_begin) * d + a;
+    const double* vp = V + (c * n_sk + col_begin) * d + a;
     double s1 = 0.0, s2 = 0.0;
-    for (int64_t k = col_begin; k + 1 < n_sk; ++k) {
-        const double tau = t[k + 1] - t[k];
-        const double x = X[(c * n_sk + k) * d + a], v = V[(c * n_sk + k) * d + a];
-        if (flow_kind == 1) {
-            double s, co;
-            sincos(tau, &s, &co);
-            const double s2t = 2.0 * s * co;  // sin(2 tau)
-            s1 += x * s + v * (1.0 - co);
-            s2 += x * x * (0.5 * tau + 0.25 * s2t) + v * v * (0.5 * tau - 0.25 * s2t) + x * v * s * s;
-        } else {
-            s1 += tau * (x + 0.5 * v * tau);
-            s2 += tau * (x * x + tau * (x * v + v * v * tau * (1.0 / 3.0)));
-        }
+    int64_t n = n_sk - 1 - col_begin;   // segments left
+    for (; n >= kMomU; n -= kMomU, tp += kMomU, xp += kMomU * d, vp += kMomU * d) {
+        double tk[kMomU + 1], x[kMomU], v[kMomU];
+#pragma unroll
+        for (int i = 0; i <= kMomU; ++i) tk[i] = tp[i];
+#pragma unroll
+        for (int i = 0; i < kMomU; ++i) { x[i] = xp[i * d]; v[i] = vp[i * d]; }
+#pragma unroll
+        for (int i = 0; i < kMomU; ++i) moment_segment<FLOW>(tk[i + 1] - tk[i], x[i], v[i], s1, s2);
     }
+    for (; n > 0; --n, ++tp, xp += d, vp += d) moment_segment<FLOW>(tp[1] - tp[0], *xp, *vp, s1, s2);
     m1[e] = s1;
     m2[e] = s2;
     if (a == 0 && Tlen) Tlen[c] = t[n_sk - 1] - t[col_begin];
@@ -1280,7 +1299,8 @@ int pdmpflux_skeleton_moments(int flow_kind, int dim, int64_t n_sk, int64_t n_ch
         p1 = d1.as<double>(); p2 = d2.as<double>(); pT = dT.as<double>();
     }
     const int64_t total = n_chains * dim;
-    moments_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(flow_kind, dim, n_sk, n_chains, col_begin, pX, pV, pt, p1, p2, pT);
+    auto kern = flow_kind == 1 ? moments_kernel<1> : moments_kernel<0>;
+    kern<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(dim, n_sk, n_chains, col_begin, pX, pV, pt, p1, p2, pT);
     CUDA_TRY(cudaGetLastError());
     g_launches.fetch_add(1);
     if (!on_device) {

@@ -473,6 +473,16 @@ struct Chain {
         dy = c2 * (pvv - pxx) - 4.0 * sc * pxv;  // v_t' H v_t - <grad U(x_t), x_t>
     }
 
+    // Compressed line model: does any active lane hold a sign-changing coordinate in slots k0 .. k0+3?  Slots past
+    // cl_n hold A = B = 0 and add max(0, 0 + t 0) = +0.0 to accumulators that are already >= +0.0, so a group that
+    // no lane uses is skipped without changing a bit (C2 keeps about 6 of the 12 slots).  The vote keeps the branch
+    // warp-uniform; a lane whose own slots are empty still runs a group some other lane needs, which adds +0.0.
+    // Teams only: the thread-per-chain kernel is issue bound and measured 5 % slower at 65536 chains with the votes.
+    __device__ __forceinline__ bool crossing_group_used(int k0) const {
+        if constexpr (!kTeamSpec) return true;
+        else return __any_sync(__activemask(), k0 < cl_n);
+    }
+
     // `sampler.rate` (always the unsigned rate): ZigZagSamplers.jl:83-86, BouncyParticleSamplers.jl:39-42,
     // ForwardEventChainMonteCarlo.jl:20-23, BoomerangSamplers.jl:38-41.  Uses Lx/Lv of the current (x, v).
     __device__ double rate_unsigned(double tt) {
@@ -506,6 +516,7 @@ struct Chain {
                 double c[4] = {0.0, 0.0, 0.0, 0.0};
 #pragma unroll
                 for (int k = 0; k < kCrossMax; ++k) {   // empty slots are A = B = 0: max(0, 0) = 0
+                    if ((k & 3) == 0 && !crossing_group_used(k)) break;
                     const double y = fma(tt, cb[k], ca[k]);
                     c[k & 3] += y + fabs(y);
                 }
@@ -612,12 +623,14 @@ struct Chain {
 #pragma unroll
                 for (int b = 0; b < B; ++b) c[b][0] = c[b][1] = c[b][2] = c[b][3] = 0.0;
 #pragma unroll
-                for (int k = 0; k < kCrossMax; ++k)
+                for (int k = 0; k < kCrossMax; ++k) {
+                    if ((k & 3) == 0 && !crossing_group_used(k)) break;
 #pragma unroll
                     for (int b = 0; b < B; ++b) {
                         const double y = fma(tt[b], cb[k], ca[k]);
                         c[b][k & 3] += y + fabs(y);
                     }
+                }
 #pragma unroll
                 for (int b = 0; b < B; ++b) {
                     double s = fma(0.5, (c[b][0] + c[b][1]) + (c[b][2] + c[b][3]), fma(tt[b], cl_be, cl_al));
@@ -1298,7 +1311,7 @@ struct Chain {
                         X[b] = mx; W[b] = mw; V[b] = mv;
                     }
                 }
-                double F[S], TOL[S], ulast = 0.0;
+                double F[S], TOL[S], U[S];
                 unsigned long long stopmask = 0ull, goodmask = 0ull;
                 bool asok[S];
 #pragma unroll
@@ -1307,13 +1320,15 @@ struct Chain {
                     const double moving = first ? (right ? s.lo : s.hi) : W[b];
                     const double lo_ = right ? moving : s.lo, hi_ = right ? s.hi : moving;
                     double mid, og, gstp;
-                    const double u = brent_golden(lo_, hi_, X[b], TOL[b], mid, og, gstp);
+                    U[b] = brent_golden(lo_, hi_, X[b], TOL[b], mid, og, gstp);
                     const bool stop = fabs(X[b] - mid) <= fma(hi_ - lo_, -0.5, TOL[b] + TOL[b]);
                     asok[b] = ((X[b] < mid) == right) & (fabs(gstp) >= TOL[b]);
-                    F[b] = -rate_unsigned(u);
-                    if (b == S - 1) ulast = u;
                     stopmask |= (unsigned long long)(stop ? 1u : 0u) << (TEAM * b + tl);   // my bits; merged below
                 }
+                rate_unsigned_n<S>(U, F);   // the S rates side by side (bit-identical to S calls of rate_unsigned)
+#pragma unroll
+                for (int b = 0; b < S; ++b) F[b] = -F[b];
+                const double ulast = U[S - 1];
                 {
                     double r1p = 0.0, r2p = 0.0, r3p = 0.0;   // the rotations of the previous block of TEAM iterations
 #pragma unroll
