@@ -18,8 +18,10 @@
 #ifndef PDMPFLUX_CUDA_H
 #define PDMPFLUX_CUDA_H
 
+#ifndef __CUDACC_RTC__ /* the run-time compiled kernels get the fixed-width types from common.cuh */
 #include <stddef.h>
 #include <stdint.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -34,7 +36,8 @@ typedef enum pdmpflux_error {
     PDMPFLUX_ERR_UNSUPPORTED = -3,        /* sampler/potential/option outside the device path (no fallback) */
     PDMPFLUX_ERR_CUDA = -4,               /* CUDA runtime error, or no device */
     PDMPFLUX_ERR_CHAIN = -5,              /* at least one chain stopped; see per-chain status */
-    PDMPFLUX_ERR_CAPACITY = -6            /* time-horizon variant: some chain needs more than `capacity` columns */
+    PDMPFLUX_ERR_CAPACITY = -6,           /* time-horizon variant: some chain needs more than `capacity` columns */
+    PDMPFLUX_ERR_COMPILE = -7             /* a source potential did not compile; pdmpflux_last_error() holds the NVRTC log */
 } pdmpflux_error;
 
 /* src/Samplers/{ZigZagSamplers,BouncyParticleSamplers,ForwardEventChainMonteCarlo,BoomerangSamplers}.jl */
@@ -53,11 +56,13 @@ typedef enum pdmpflux_sampler_kind {
  *   BANANA               -                      test/test_config.jl:33-36
  *   BANANA_README_SCALAR -                      README.md:62-65 (scalar "gradient" broadcast to all coords)
  *   LOGREG               n, sigma0, X[n*d] row-major, y[n]
+ *   SOURCE               p[n_params]            user-written CUDA source (pdmpflux_potential_create_source)
  * (A dense-precision Gaussian is not offered: the only "slanted" Gaussian BASELINE names is GAUSS_EQUICORR.)
  */
 typedef enum pdmpflux_potential_kind {
     PDMPFLUX_GAUSS_STD = 0, PDMPFLUX_GAUSS_DIAG = 1, PDMPFLUX_GAUSS_EQUICORR = 2, PDMPFLUX_BANANA = 3,
-    PDMPFLUX_BANANA_README_SCALAR = 4, PDMPFLUX_LOGREG = 5
+    PDMPFLUX_BANANA_README_SCALAR = 4, PDMPFLUX_LOGREG = 5,
+    PDMPFLUX_SOURCE = 6 /* created by pdmpflux_potential_create_source only */
 } pdmpflux_potential_kind;
 
 /* How d/dt of the rate is obtained on the time grid: JVP = analytic (what AD_backend="ForwardDiff" computes,
@@ -131,6 +136,7 @@ typedef struct pdmpflux_potential_s* pdmpflux_potential_t;
 typedef struct pdmpflux_sampler_s* pdmpflux_sampler_t;
 typedef struct pdmpflux_chains_s* pdmpflux_chains_t;
 
+#ifndef __CUDACC_RTC__ /* host entry points: not part of the run-time compiled kernels */
 int pdmpflux_version(void);
 const char* pdmpflux_last_error(void);
 int pdmpflux_device_count(int* count);
@@ -140,6 +146,36 @@ int pdmpflux_set_device(int device);
 int pdmpflux_potential_create(int kind, int dim, const double* params, int64_t n_params,
                               pdmpflux_potential_t* out);
 int pdmpflux_potential_destroy(pdmpflux_potential_t pot);
+
+/* A potential written by the user in CUDA C++ (the closest thing to the reference's arbitrary `grad U` closure).
+ * `source` defines one struct at global scope with the members of the built-in plugins (csrc/potentials.cuh):
+ *
+ *   struct UserPotential {   // U = sum_i log cosh(s_i x_i) + c/2 (sum_i x_i)^2 ; params = s[0..d-1], c
+ *       static constexpr int K = 1;                                        // number of linear functionals, 0 <= K <= 8
+ *       __device__ static void accum(const pdmpflux::PotParams&, int i, double xi, double* acc) { acc[0] += xi; }
+ *       __device__ static double grad(const pdmpflux::PotParams& pp, int i, double xi, const double* Lx) {
+ *           const double s = pp.vec[i];
+ *           return s * tanh(s * xi) + pp.vec[pp.n - 1] * Lx[0];
+ *       }
+ *       __device__ static void eval(const pdmpflux::PotParams& pp, int i, double xi, double di, const double* Lx,
+ *                                   const double* Ld, double& g, double& hd) {
+ *           const double s = pp.vec[i], th = tanh(s * xi), c = pp.vec[pp.n - 1];
+ *           g = s * th + c * Lx[0];
+ *           hd = s * s * (1.0 - th * th) * di + c * Ld[0];
+ *       }
+ *   };
+ *
+ *   accum(pp, i, xi, acc)               acc[k] += contribution of coordinate i to the linear functional L_k(x).  It MUST
+ *                                       be linear in xi: along the flow the kernels evaluate L(x_t) as a L(x) + b L(v).
+ *   grad(pp, i, xi, Lx)                 (grad U(x))_i, given x_i and the functionals Lx = L(x)
+ *   eval(pp, i, xi, di, Lx, Ld, g, hd)  g = (grad U(x))_i and hd = (H(x) dir)_i, where dir_i = di and Ld = L(dir)
+ *
+ * pp.vec is a device copy of params[0 .. n_params-1] and pp.n = n_params.  The gradient may depend on the whole vector
+ * only through the K functionals.  The source is compiled with NVRTC (bound at run time; ERR_UNSUPPORTED without it):
+ * a contract check here (ERR_COMPILE with the log, lines numbered as `user_potential(<line>)`), the kernels when a
+ * sampler is created.  Every sampler kind runs it on the generic kernel; pdmpflux_rv_diagnostic does not (no U value). */
+int pdmpflux_potential_create_source(int dim, const char* source, const double* params, int64_t n_params,
+                                     pdmpflux_potential_t* out);
 
 /* replaces ZigZag(dim, grad U; kw...) / BPS / ForwardECMC / Boomerang constructors */
 int pdmpflux_sampler_create(int sampler_kind, int dim, pdmpflux_potential_t pot, const pdmpflux_config* cfg,
@@ -288,11 +324,14 @@ int pdmpflux_host_free(void* ptr);
 
 /* number of kernel launches issued by this library in this process (bench.py's gpu_launches) */
 int64_t pdmpflux_launch_count(void);
+/* number of NVRTC compiles of source potentials in this process (contract checks and kernels; cached ones not counted) */
+int64_t pdmpflux_jit_compile_count(void);
 
 /* bytes that crossed PCIe in the last host-buffer sample_skeleton call of this process (initial states in; history
  * out -- for Zig-Zag the V rows travel as sign bits and are rebuilt on the host, so this is less than the size of
  * the history).  bench.py's e2e.{h2d,d2h}_bytes_per_step. */
 int pdmpflux_last_transfer_bytes(int64_t* h2d, int64_t* d2h);
+#endif /* __CUDACC_RTC__ */
 
 #ifdef __cplusplus
 }

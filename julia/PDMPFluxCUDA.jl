@@ -10,7 +10,7 @@ module PDMPFluxCUDA
 import PDMPFlux
 import PDMPFlux: PDMPHistory, sample_skeleton, sample_from_skeleton, sample, RV_diagnostic,
                  sample_skeleton_with_diagnostic
-export CuPotential, GaussStd, GaussDiag, GaussEquicorr, Banana, BananaReadmeScalar, LogReg, CuPDMP, CuHistoryBatch,
+export CuPotential, GaussStd, GaussDiag, GaussEquicorr, Banana, BananaReadmeScalar, LogReg, CudaPotential, CuPDMP, CuHistoryBatch,
        moments_reduce, CuComm, comm_unique_id, moments_allreduce!
 
 const LIB = get(ENV, "PDMPFLUX_CUDA_LIB", joinpath(@__DIR__, "..", "pdmpflux.jl_b200", "lib", "libpdmpflux_cuda.so"))
@@ -34,6 +34,7 @@ function check(rc::Integer)
     msg = last_error()
     rc == -1 && throw(ArgumentError(msg))          # PDMPFLUX_ERR_ARGUMENT
     rc == -2 && throw(DimensionMismatch(msg))      # PDMPFLUX_ERR_DIMENSION_MISMATCH
+    rc == -7 && throw(ErrorException("CudaPotential did not compile:\n" * msg))   # PDMPFLUX_ERR_COMPILE (NVRTC log)
     error("libpdmpflux_cuda ($rc): $msg")          # unsupported / CUDA / chain failure: there is no CPU fallback
 end
 function __init__()
@@ -45,7 +46,9 @@ end
 struct CuPotential
     kind::Int32
     params::Vector{Float64}
+    source::Union{Nothing,String}   # kind 6 (PDMPFLUX_SOURCE): user CUDA source
 end
+CuPotential(kind::Integer, params::Vector{Float64}) = CuPotential(Int32(kind), params, nothing)
 GaussStd() = CuPotential(0, Float64[])
 GaussDiag(p::AbstractVector) = CuPotential(1, collect(Float64, p))
 GaussEquicorr(rho::Real) = CuPotential(2, [Float64(rho)])
@@ -55,6 +58,15 @@ BananaReadmeScalar() = CuPotential(4, Float64[])
 passed row-major, i.e. as the memory of `permutedims(X)`."
 LogReg(X::AbstractMatrix, y::AbstractVector, sigma0::Real) =
     CuPotential(5, vcat(Float64(size(X, 1)), Float64(sigma0), vec(permutedims(Matrix{Float64}(X))), Vector{Float64}(y)))
+"""
+    CudaPotential(source, params=Float64[])
+
+A potential written in CUDA C++: `source` defines `struct UserPotential` (K linear functionals, `accum`, `grad`,
+`eval`; the contract is stated in include/pdmpflux_cuda.h above `pdmpflux_potential_create_source`) and `params` are
+`pp.vec[0 .. pp.n-1]` on the device.  Compiled at run time with NVRTC when the sampler is constructed.
+"""
+CudaPotential(source::AbstractString, params::AbstractVector=Float64[]) =
+    CuPotential(Int32(6), collect(Float64, params), String(source))
 
 "A sampler living on the GPU: what the reference constructors return when the second argument is a `CuPotential`."
 mutable struct CuPDMP
@@ -69,8 +81,13 @@ deriv_mode(ad::String) = ad in ("", "Undefined", "FiniteDiff") ? Int32(1) :
 function CuPDMP(kind, dim::Int, pot::CuPotential, cfg::CConfig; kappa::Union{Nothing,Vector{Float64}}=nothing)
     dim <= 0 && throw(ArgumentError("dimension dim must be positive. Current value: $dim"))
     hp = Ref{Ptr{Cvoid}}(C_NULL)
-    check(ccall((:pdmpflux_potential_create, LIB), Cint, (Cint, Cint, Ptr{Float64}, Int64, Ref{Ptr{Cvoid}}),
-                pot.kind, dim, pot.params, length(pot.params), hp))
+    if pot.source === nothing
+        check(ccall((:pdmpflux_potential_create, LIB), Cint, (Cint, Cint, Ptr{Float64}, Int64, Ref{Ptr{Cvoid}}),
+                    pot.kind, dim, pot.params, length(pot.params), hp))
+    else
+        check(ccall((:pdmpflux_potential_create_source, LIB), Cint, (Cint, Cstring, Ptr{Float64}, Int64, Ref{Ptr{Cvoid}}),
+                    dim, pot.source, pot.params, length(pot.params), hp))
+    end
     hs = Ref{Ptr{Cvoid}}(C_NULL)
     rc = if kappa === nothing
         ccall((:pdmpflux_sampler_create, LIB), Cint, (Cint, Cint, Ptr{Cvoid}, Ref{CConfig}, Ref{Ptr{Cvoid}}),

@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # PDMPFLUX_CUDA_LIB points at another build of the same library (A/B experiments); the default is the in-tree build
 LIB_PATH = os.environ.get("PDMPFLUX_CUDA_LIB") or os.path.join(_HERE, "lib", "libpdmpflux_cuda.so")
 
-OK, ERR_ARGUMENT, ERR_DIMENSION_MISMATCH, ERR_UNSUPPORTED, ERR_CUDA, ERR_CHAIN, ERR_CAPACITY = 0, -1, -2, -3, -4, -5, -6
+OK, ERR_ARGUMENT, ERR_DIMENSION_MISMATCH, ERR_UNSUPPORTED, ERR_CUDA, ERR_CHAIN, ERR_CAPACITY, ERR_COMPILE = 0, -1, -2, -3, -4, -5, -6, -7
 
 
 class ArgumentError(ValueError):
@@ -31,6 +31,11 @@ class UnsupportedError(NotImplementedError):
 
 class CudaError(RuntimeError):
     pass
+
+
+class CompileError(ValueError):
+    """The CUDA source of a CudaPotential did not compile; the message is the NVRTC log (lines of the user's text
+    appear as `user_potential(<line>)`)."""
 
 
 class CapacityError(RuntimeError):
@@ -74,6 +79,7 @@ SIGNATURES = {
     "pdmpflux_device_count": (C.c_int, [C.POINTER(C.c_int)]),
     "pdmpflux_set_device": (C.c_int, [C.c_int]),
     "pdmpflux_potential_create": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
+    "pdmpflux_potential_create_source": (C.c_int, [C.c_int, C.c_char_p, C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]),
     "pdmpflux_potential_destroy": (C.c_int, [C.c_void_p]),
     "pdmpflux_sampler_create": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.POINTER(Config), C.POINTER(C.c_void_p)]),
     "pdmpflux_sampler_create_sticky": (C.c_int, [C.c_int, C.c_void_p, C.POINTER(Config), C.c_void_p, C.POINTER(C.c_void_p)]),
@@ -121,6 +127,7 @@ SIGNATURES = {
     "pdmpflux_host_alloc": (C.c_int, [C.POINTER(C.c_void_p), C.c_size_t]),
     "pdmpflux_host_free": (C.c_int, [C.c_void_p]),
     "pdmpflux_launch_count": (C.c_int64, []),
+    "pdmpflux_jit_compile_count": (C.c_int64, []),
     "pdmpflux_last_transfer_bytes": (C.c_int, [C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
 }
 
@@ -165,4 +172,6 @@ def check(rc, status=None):
         raise ChainError(msg, status)
     if rc == ERR_CAPACITY:
         raise CapacityError(msg)
+    if rc == ERR_COMPILE:
+        raise CompileError(msg)
     raise CudaError(msg)

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -21,6 +22,7 @@
 #endif
 
 #include "common.cuh"
+#include "jit.cuh"
 #include "launch.cuh"
 
 using namespace pdmpflux;
@@ -68,6 +70,7 @@ struct pdmpflux_potential_s {
     int kind = 0, dim = 0;
     PotParams pp{};
     DevBuf params;
+    std::string source;  // PDMPFLUX_SOURCE: the user's CUDA text (jit.cu)
 };
 
 // Device slabs of the host-buffer pipeline, cached in the sampler handle so that repeated sample_skeleton calls do
@@ -132,6 +135,7 @@ struct pdmpflux_chains_s {
 namespace {
 
 // Team widths built: 1, 8, 32 for everything; 4 only for the register-resident Zig-Zag x Brent kernels (launch.cuh).
+int default_team(int d, int64_t n_chains, bool zz_brent_fast);
 int pick_team(int d, int64_t n_chains, bool zz_brent_fast, int sampler) {
     if (const char* e = std::getenv("PDMPFLUX_TEAM")) {
         const int t = std::atoi(e);  // only the team widths launch_for_sampler instantiates
@@ -141,6 +145,9 @@ int pick_team(int d, int64_t n_chains, bool zz_brent_fast, int sampler) {
         if (t == PDMPFLUX_EXTRA_TEAM) return t;
 #endif
     }
+    return default_team(d, n_chains, zz_brent_fast);
+}
+int default_team(int d, int64_t n_chains, bool zz_brent_fast) {
     // Measured on B200 (profiles/): thread-per-chain wins for small d once there are enough chains to occupy the
     // SMs; 8 lanes per chain win for d up to a few hundred (fewer shuffle stages than a full warp, 4 chains share a
     // warp's instruction stream); a warp per chain beyond that (and whenever the shared-memory state would not fit).
@@ -157,6 +164,19 @@ int pick_team(int d, int64_t n_chains, bool zz_brent_fast, int sampler) {
     // almost every event, so the whole warp pays the d-normal pass every time.)
     if (d <= 256) return 8;
     return 32;
+}
+
+// widen the team until the per-thread-owned shared-memory columns of a block (x, v, Zig-Zag x Brent A / B, moments,
+// sticky flags; ForwardECMC scratch goes to global memory when it is large) leave room for a second block
+int widen_team(int team, int sampler, int path, int d, bool zz_brent_fast) {
+    auto vectors_bytes = [&](int team) {
+        const int bt_ = block_threads_rt(team, sampler, path);
+        const size_t nv = (zz_brent_fast && team > 1 && brent_reg_nw(sampler, path, team, (d + team - 1) / team) <= 0) ? 4 : 2;
+        return (nv + 2 /* fused moments may be enabled later */ + (sampler == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) *
+               (size_t)((d + team - 1) / team) * bt_ * sizeof(double);
+    };
+    while (team < 32 && vectors_bytes(team) > 110 * 1024) team = team < 8 ? 8 : 32;
+    return team;
 }
 
 // `rows`: optional separate placement of the X / V rows (host pipeline: rows go through narrow double-buffered
@@ -225,7 +245,11 @@ int launch(pdmpflux_chains_s* ch, int64_t n_events, const pdmpflux_history* h, i
     cudaError_t e;
     const size_t smem_launch = ch->smem + (ch->moments ? 2 * (size_t)ch->vec_elems * sizeof(double) : 0);
     if (smem_launch > 227 * 1024) return fail(PDMPFLUX_ERR_UNSUPPORTED, "fused moments: shared memory exhausted for this dimension");
-    if (s->pot->kind == PDMPFLUX_LOGREG) {
+    if (s->pot->kind == PDMPFLUX_SOURCE) {
+        const int rc = jit_launch(s->pot->source, s->kind, ch->team, p, ch->grid, smem_launch, stream);
+        if (rc != PDMPFLUX_OK) return rc;
+        e = cudaSuccess;
+    } else if (s->pot->kind == PDMPFLUX_LOGREG) {
         p.vec32 = 0; p.bulk_rows = 0;
         // One CTA per SM (384 threads, 168 registers): with more CTAs of four chains than SMs, the first wave starts on
         // chains 0 .. 4 grid - 1 and every warp pulls its next chain from a work queue when its own is done.
@@ -432,6 +456,7 @@ extern "C" {
 int pdmpflux_version(void) { return PDMPFLUX_VERSION; }
 const char* pdmpflux_last_error(void) { return g_err.c_str(); }
 int64_t pdmpflux_launch_count(void) { return g_launches.load(); }
+int64_t pdmpflux_jit_compile_count(void) { return jit_compile_count(); }
 int pdmpflux_last_transfer_bytes(int64_t* h2d, int64_t* d2h) {
     if (h2d) *h2d = g_h2d_bytes.load();
     if (d2h) *d2h = g_d2h_bytes.load();
@@ -497,10 +522,36 @@ int pdmpflux_potential_create(int kind, int dim, const double* params, int64_t n
         pot->pp.n = n;
         pot->pp.inv_s2 = 1.0 / (s0 * s0);
     } break;
+    case PDMPFLUX_SOURCE:
+        rc = fail(PDMPFLUX_ERR_ARGUMENT, "PDMPFLUX_SOURCE potentials carry CUDA source: create them with pdmpflux_potential_create_source");
+        break;
     default: rc = fail(PDMPFLUX_ERR_ARGUMENT, "unknown potential kind " + std::to_string(kind));
     }
     if (rc != PDMPFLUX_OK) { delete pot; return rc; }
     *out = pot;
+    return PDMPFLUX_OK;
+}
+
+int pdmpflux_potential_create_source(int dim, const char* source, const double* params, int64_t n_params,
+                                     pdmpflux_potential_t* out) {
+    if (!out) return fail(PDMPFLUX_ERR_ARGUMENT, "out is NULL");
+    *out = nullptr;
+    if (dim <= 0) return fail(PDMPFLUX_ERR_ARGUMENT, "dimension dim must be positive. Current value: " + std::to_string(dim));
+    if (!source) return fail(PDMPFLUX_ERR_ARGUMENT, "source is NULL");
+    if (n_params < 0 || (n_params > 0 && !params)) return fail(PDMPFLUX_ERR_ARGUMENT, "params must hold n_params >= 0 doubles");
+    auto pot = std::make_unique<pdmpflux_potential_s>();
+    pot->kind = PDMPFLUX_SOURCE; pot->dim = dim; pot->source = source;
+    // the contract check runs before any CUDA call: bad source fails here, with or without a device
+    const int rc = jit_check_source(pot->source);
+    if (rc != PDMPFLUX_OK) return rc;
+    if (n_params > 0) {
+        if (pot->params.alloc(sizeof(double) * (size_t)n_params) != cudaSuccess ||
+            cudaMemcpy(pot->params.p, params, sizeof(double) * (size_t)n_params, cudaMemcpyHostToDevice) != cudaSuccess)
+            return fail(PDMPFLUX_ERR_CUDA, "source potential parameter upload failed (is a CUDA device present?)");
+        pot->pp.vec = pot->params.as<double>();
+    }
+    pot->pp.n = n_params;
+    *out = pot.release();
     return PDMPFLUX_OK;
 }
 int pdmpflux_potential_destroy(pdmpflux_potential_t pot) { delete pot; return PDMPFLUX_OK; }
@@ -535,6 +586,15 @@ static int sampler_create_impl(int kind, int dim, pdmpflux_potential_t pot, cons
     if (kind == PDMPFLUX_FECMC && dim < 2)
         return fail(PDMPFLUX_ERR_ARGUMENT, "The dimension must be at least 2 to use the ForwardEventChain. Got dimension " + std::to_string(dim));
     if (!(cfg->tmax >= 0.0) || !std::isfinite(cfg->tmax)) return fail(PDMPFLUX_ERR_ARGUMENT, "tmax must be finite and >= 0");
+    if (pot->kind == PDMPFLUX_SOURCE) {
+        // compile every team width the default policy can pick for this (kind, dim) -- the kernel is the generic one
+        // whatever the config -- before any CUDA call, so that source errors surface here even without a device
+        for (int64_t n_chains : {int64_t(1), INT64_MAX}) {
+            const int team = widen_team(default_team(dim, n_chains, false), kind, kPathGeneric, dim, false);
+            const int rc = jit_prepare(pot->source, kind, team);
+            if (rc != PDMPFLUX_OK) return rc;
+        }
+    }
     auto s = new pdmpflux_sampler_s();
     s->kind = kind; s->dim = dim; s->cfg = *cfg; s->pot = pot;
     normalise_config(kind, dim, s->cfg);
@@ -590,17 +650,12 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
     const bool logreg = s->pot->kind == PDMPFLUX_LOGREG;
     ch->path = select_path(s->kind, s->pot->kind, s->cfg.grid_size, s->cfg.vectorized_bound, s->cfg.deriv_mode);
     if (const char* e = std::getenv("PDMPFLUX_FORCE_GENERIC")) { if (std::atoi(e)) ch->path = kPathGeneric; }
-    ch->team = pick_team(d, n_chains, s->kind == PDMPFLUX_ZIGZAG && ch->path == kPathFastBrent && !logreg, s->kind);
-    // widen the team until the per-thread-owned shared-memory columns of a block (x, v, Zig-Zag x Brent A / B, moments,
-    // sticky flags; ForwardECMC scratch goes to global memory when it is large) leave room for a second block
     const bool zz_brent_fast = s->kind == PDMPFLUX_ZIGZAG && ch->path == kPathFastBrent && !logreg;
-    auto vectors_bytes = [&](int team) {
-        const int bt_ = block_threads_rt(team, s->kind, ch->path);
-        const size_t nv = (zz_brent_fast && team > 1 && brent_reg_nw(s->kind, ch->path, team, (d + team - 1) / team) <= 0) ? 4 : 2;
-        return (nv + 2 /* fused moments may be enabled later */ + (s->kind == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) *
-               (size_t)((d + team - 1) / team) * bt_ * sizeof(double);
-    };
-    while (ch->team < 32 && vectors_bytes(ch->team) > 110 * 1024) ch->team = ch->team < 8 ? 8 : 32;
+    ch->team = widen_team(pick_team(d, n_chains, zz_brent_fast, s->kind), s->kind, ch->path, d, zz_brent_fast);
+    if (s->pot->kind == PDMPFLUX_SOURCE) {  // a width sampler_create did not compile (PDMPFLUX_TEAM): compile it now
+        const int rc = jit_prepare(s->pot->source, s->kind, ch->team);
+        if (rc != PDMPFLUX_OK) return rc;
+    }
     ch->n_own = (d + ch->team - 1) / ch->team;
     const int bt = block_threads_rt(ch->team, s->kind, ch->path);   // threads per block of the kernel that will run
     const int cpb = bt / ch->team;
@@ -1317,6 +1372,8 @@ int pdmpflux_rv_diagnostic(pdmpflux_potential_t pot, int flow_kind, int64_t n_sk
                            double* rv, int32_t on_device, void* stream_) {
     if (!pot || !X || !V || !t || !rv || n_sk <= 0 || ld_sk < n_sk || n_chains <= 0)
         return fail(PDMPFLUX_ERR_ARGUMENT, "invalid argument");
+    if (pot->kind == PDMPFLUX_SOURCE)
+        return fail(PDMPFLUX_ERR_UNSUPPORTED, "RV_diagnostic needs U(x), which a source potential does not define (it gives grad U only)");
     if (B < 0) return fail(PDMPFLUX_ERR_ARGUMENT, "B must be non-negative");  // diagnostic.jl:49-51
     if (flow_kind != 0 && flow_kind != 1) return fail(PDMPFLUX_ERR_ARGUMENT, "flow_kind must be 0 (linear) or 1 (rotation)");
     int ndev = 0;

@@ -1,7 +1,15 @@
 // Shared declarations for the thinning kernels: launch parameters, team (sub-warp) collectives.
 #pragma once
+#ifdef __CUDACC_RTC__  // run-time compiled (jit.cu): NVRTC has the CUDA built-ins but no C++ library headers
+typedef unsigned char uint8_t;
+typedef int int32_t;
+typedef unsigned int uint32_t;
+typedef long int64_t;            // LP64, as <cstdint> on the Linux hosts the library is built on
+typedef unsigned long uint64_t;
+#else
 #include <cstdint>
 #include <cuda_runtime.h>
+#endif
 #include <math_constants.h>
 
 #include "../../include/pdmpflux_cuda.h"

@@ -10,7 +10,11 @@
 //   N slot j : call j>>1, Box-Muller: sqrt(-2 log u1) * (j&1 ? sin : cos)(2 pi u2)
 // The same specification is restated for the CPU in oracle/pdmp_draws.h (test infrastructure).
 #pragma once
+#ifdef __CUDACC_RTC__
+#include "common.cuh"  // fixed-width types
+#else
 #include <cstdint>
+#endif
 
 namespace pdmpflux {
 

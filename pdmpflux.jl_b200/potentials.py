@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _lib
 
-GAUSS_STD, GAUSS_DIAG, GAUSS_EQUICORR, BANANA, BANANA_README_SCALAR, LOGREG = range(6)
+GAUSS_STD, GAUSS_DIAG, GAUSS_EQUICORR, BANANA, BANANA_README_SCALAR, LOGREG, SOURCE = range(7)
 
 
 class Potential:
@@ -84,3 +84,31 @@ class LogReg(Potential):
         if d != dim or self.y.shape != (n,):
             raise _lib.DimensionMismatch("LogReg design matrix does not match dim")
         return np.concatenate([[float(n), self.sigma0], self.X.ravel(), self.y])
+
+
+class CudaPotential(Potential):
+    """A potential written in CUDA C++: `source` defines `struct UserPotential` with the members of the built-in
+    plugins (K linear functionals, accum, grad, eval; see include/pdmpflux_cuda.h or INTEGRATION.md), and `params`
+    becomes `pp.vec[0 .. pp.n - 1]` on the device.  The source is compiled at run time with NVRTC: a contract check
+    when each sampler is built (CompileError carries the compiler log) and the sampler's kernels right after it.
+    Compiled kernels are cached per process by source, so samplers that only change `params` do not compile again.
+
+    `accum` must be linear in x_i; the library cannot check it.  Every sampler runs a CudaPotential on its generic
+    kernel; RV_diagnostic does not (the contract has no U value)."""
+    kind = SOURCE
+
+    def __init__(self, source, params=()):
+        if not isinstance(source, str):
+            raise TypeError("CudaPotential source must be a str of CUDA C++")
+        self.source = source
+        self.p = np.ascontiguousarray(params, dtype=np.float64).ravel()
+
+    def params(self, dim):
+        return self.p
+
+    def _create(self, dim):
+        h = C.c_void_p()
+        _lib.check(_lib.lib().pdmpflux_potential_create_source(int(dim), self.source.encode(),
+                                                               self.p.ctypes.data if self.p.size else None,
+                                                               self.p.size, C.byref(h)))
+        return h
