@@ -117,7 +117,7 @@ struct pdmpflux_chains_s {
     int64_t n_chains = 0, chain_offset = 0, event0 = 0;
     uint64_t seed = 0;
     int team = 32, n_own = 0, scratch_in_smem = 1, path = 0, vec_elems = 0, dpad = 0;
-    int brent_nw = 0;   // Zig-Zag x Brent line-model variant (brent_reg_nw), fixed when the chains are created
+    int brent_nw = kLineShared;   // Zig-Zag x Brent line model (brent_line_model), fixed when the chains are created
     size_t smem = 0;
     unsigned grid = 0;
     int64_t n_groups = 0;   // groups of chains (one block's worth); grid < n_groups: persistent blocks walk over the groups
@@ -134,16 +134,15 @@ struct pdmpflux_chains_s {
 
 namespace {
 
-// Team widths built: 1, 8, 32 for everything; 4 only for the register-resident Zig-Zag x Brent kernels (launch.cuh).
+// Team widths built: 1, 8, 32 (launch.cuh: launch_for_sampler).
 int default_team(int d, int64_t n_chains, bool zz_brent_fast);
-int pick_team(int d, int64_t n_chains, bool zz_brent_fast, int sampler) {
+int pick_team(int d, int64_t n_chains, bool zz_brent_fast) {
     if (const char* e = std::getenv("PDMPFLUX_TEAM")) {
-        const int t = std::atoi(e);  // only the team widths launch_for_sampler instantiates
-        if (t == 1 || t == 8 || t == 32) return t;
-        if (t == 4 && zz_brent_fast && d <= 64) return t;
-#ifdef PDMPFLUX_EXTRA_TEAM
-        if (t == PDMPFLUX_EXTRA_TEAM) return t;
-#endif
+        // only a width with a kernel for this shape: thread-per-chain Zig-Zag x Brent packs coordinate indices into 6
+        // bits (chain.cuh: classify_line), so it is built for d <= 64 (widen_team's shared-memory budget already widens
+        // it above d = 55; this check does not depend on that budget)
+        const int t = std::atoi(e);
+        if (t == 8 || t == 32 || (t == 1 && !(zz_brent_fast && d > 64))) return t;
     }
     return default_team(d, n_chains, zz_brent_fast);
 }
@@ -168,12 +167,13 @@ int default_team(int d, int64_t n_chains, bool zz_brent_fast) {
 
 // widen the team until the per-thread-owned shared-memory columns of a block (x, v, Zig-Zag x Brent A / B, moments,
 // sticky flags; ForwardECMC scratch goes to global memory when it is large) leave room for a second block
-int widen_team(int team, int sampler, int path, int d, bool zz_brent_fast) {
+int widen_team(int team, int sampler, int path, int d) {
     auto vectors_bytes = [&](int team) {
         const int bt_ = block_threads_rt(team, sampler, path);
-        const size_t nv = (zz_brent_fast && team > 1 && brent_reg_nw(sampler, path, team, (d + team - 1) / team) <= 0) ? 4 : 2;
+        const int n_own = (d + team - 1) / team;
+        const size_t nv = state_vectors(sampler, path, team, brent_line_model(sampler, path, team, n_own));
         return (nv + 2 /* fused moments may be enabled later */ + (sampler == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) *
-               (size_t)((d + team - 1) / team) * bt_ * sizeof(double);
+               (size_t)n_own * bt_ * sizeof(double);
     };
     while (team < 32 && vectors_bytes(team) > 110 * 1024) team = team < 8 ? 8 : 32;
     return team;
@@ -590,7 +590,7 @@ static int sampler_create_impl(int kind, int dim, pdmpflux_potential_t pot, cons
         // compile every team width the default policy can pick for this (kind, dim) -- the kernel is the generic one
         // whatever the config -- before any CUDA call, so that source errors surface here even without a device
         for (int64_t n_chains : {int64_t(1), INT64_MAX}) {
-            const int team = widen_team(default_team(dim, n_chains, false), kind, kPathGeneric, dim, false);
+            const int team = widen_team(default_team(dim, n_chains, false), kind, kPathGeneric, dim);
             const int rc = jit_prepare(pot->source, kind, team);
             if (rc != PDMPFLUX_OK) return rc;
         }
@@ -651,7 +651,7 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
     ch->path = select_path(s->kind, s->pot->kind, s->cfg.grid_size, s->cfg.vectorized_bound, s->cfg.deriv_mode);
     if (const char* e = std::getenv("PDMPFLUX_FORCE_GENERIC")) { if (std::atoi(e)) ch->path = kPathGeneric; }
     const bool zz_brent_fast = s->kind == PDMPFLUX_ZIGZAG && ch->path == kPathFastBrent && !logreg;
-    ch->team = widen_team(pick_team(d, n_chains, zz_brent_fast, s->kind), s->kind, ch->path, d, zz_brent_fast);
+    ch->team = widen_team(pick_team(d, n_chains, zz_brent_fast), s->kind, ch->path, d);
     if (s->pot->kind == PDMPFLUX_SOURCE) {  // a width sampler_create did not compile (PDMPFLUX_TEAM): compile it now
         const int rc = jit_prepare(s->pot->source, s->kind, ch->team);
         if (rc != PDMPFLUX_OK) return rc;
@@ -668,10 +668,10 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
         ch->vec_elems = cpb * ch->dpad;
     }
     const size_t vec_bytes = (size_t)ch->vec_elems * sizeof(double);
-    ch->brent_nw = brent_reg_nw(s->kind, ch->path, ch->team, ch->n_own);
-    const size_t nvec = (s->kind == PDMPFLUX_ZIGZAG && ch->path == kPathFastBrent && ch->team > 1 && ch->brent_nw <= 0) ? 4 : 2;
+    ch->brent_nw = brent_line_model(s->kind, ch->path, ch->team, ch->n_own);
+    const size_t nvec = state_vectors(s->kind, ch->path, ch->team, ch->brent_nw);
     ch->smem = (nvec + (s->kind == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) * vec_bytes;
-    const size_t list_slack = ch->brent_nw < 0 ? 16 * sizeof(double) : 0;   // transposed Brent: unconditional reads of the 12-slot list
+    const size_t list_slack = ch->brent_nw == kLineTransposed ? 16 * sizeof(double) : 0;   // transposed Brent: unconditional reads of the 12-slot list
     if (s->kind == PDMPFLUX_FECMC) {
         if ((nvec + 3) * vec_bytes <= 64 * 1024) { ch->scratch_in_smem = 1; ch->smem = (nvec + 3) * vec_bytes; }
         else {

@@ -60,20 +60,21 @@ extern __shared__ __align__(128) double g_smem[];
 // whose rate changes sign inside the bound's bracket (see Chain::classify_line)
 constexpr int kCrossMax = 12;
 
-// NW > 0 (Zig-Zag + kPathFastBrent only): compile-time capacity of the owned-coordinate loops; the line model
-// (A_j, B_j) of the owned coordinates then lives in registers (slots >= n_own hold A = B = 0) and the ~40 rate
-// evaluations of a Brent bound touch neither shared memory nor any loop counter.
-template <int TEAM, int SAMPLER, int POT, int PATH, int NW = 0>
+// NW (Zig-Zag + kPathFastBrent only) is the line model of common.cuh.  kLineRegs: compile-time capacity of the
+// owned-coordinate loops; the line model (A_j, B_j) of the owned coordinates then lives in registers (slots >= n_own
+// hold A = B = 0) and the ~40 rate evaluations of a Brent bound touch neither shared memory nor any loop counter.
+template <int TEAM, int SAMPLER, int POT, int PATH, int NW = kLineShared>
 struct Chain {
     using P = Pot<POT>;
     static constexpr bool kFast = (PATH != kPathGeneric);
-    static constexpr bool kRegLine = (NW > 0);
-    static constexpr int NWW = NW > 0 ? NW : 1;
-    static_assert(NW == 0 || (SAMPLER == PDMPFLUX_ZIGZAG && PATH == kPathFastBrent), "NW is a Zig-Zag x Brent option");
-    // NW < 0: "transposed" team Brent -- every lane of the team keeps the chain's compressed line model and evaluates
-    // ONE abscissa of a speculative batch of TEAM Brent iterations (see build_bound_brent)
-    static constexpr bool kTeamSpec = (NW < 0);
-    static_assert(!kTeamSpec || (TEAM > 1 && TEAM < 32), "transposed Brent: teams of 4 or 8 lanes");
+    static_assert(NW == kLineShared || NW == kLineTransposed || NW == kLineRegs, "NW is one of the kLine* models");
+    static constexpr bool kRegLine = (NW == kLineRegs);
+    static constexpr int NWW = kRegLine ? kLineRegs : 1;
+    static_assert(NW == kLineShared || (SAMPLER == PDMPFLUX_ZIGZAG && PATH == kPathFastBrent), "NW is a Zig-Zag x Brent option");
+    // kLineTransposed: "transposed" team Brent -- every lane of the team keeps the chain's compressed line model and
+    // evaluates ONE abscissa of a speculative batch of TEAM Brent iterations (see build_bound_brent)
+    static constexpr bool kTeamSpec = (NW == kLineTransposed);
+    static_assert(!kTeamSpec || TEAM == 8, "transposed Brent: teams of 8 lanes");
     static constexpr int NS = P::kSpecial;
     static constexpr int K = P::K;
     static constexpr int KK = K > 0 ? K : 1;
@@ -110,7 +111,7 @@ struct Chain {
     double cl_al, cl_be;      // compressed line model: sum of A_i, B_i over the coordinates that are active on the whole bracket
     int cl_n;                 // ... number of sign-changing coordinates kept in ca / cb (unused slots hold 0); > kCrossMax: not compressed
     double ca[kCompressed ? kCrossMax : 1], cb[kCompressed ? kCrossMax : 1];   // registers: only indexed by unrolled loops
-    double ra[NWW], rb[NWW];  // NW > 0: A_j, B_j of the owned coordinates (registers: only indexed by unrolled loops)
+    double ra[NWW], rb[NWW];  // kRegLine: A_j, B_j of the owned coordinates (registers: only indexed by unrolled loops)
     double la, lb;          // BPS/FECMC: a = sum A_i, b = sum B_i over the affine coordinates
     double pxx, pxv, pvv;   // Boomerang: <Px,x>, <Px,v>, <Pv,v>
 
@@ -392,7 +393,7 @@ struct Chain {
         } else if constexpr (kZZ) {
             if constexpr (kRegLine) {
 #pragma unroll
-                for (int j = 0; j < NW; ++j) {
+                for (int j = 0; j < kLineRegs; ++j) {
                     double A = 0.0, B = 0.0;  // A = B = 0 contributes max(0, 0) = 0 for unowned / special / padding slots
                     if (j < nown && owns(j) && coord(j) >= NS) {
                         const double vi = VS(j);
@@ -494,7 +495,7 @@ struct Chain {
             // max(0, y) = (y + |y|) / 2 exactly in binary floating point; four accumulators, everything in registers
             double acc[4] = {0.0, 0.0, 0.0, 0.0};
 #pragma unroll
-            for (int j = 0; j < NW; ++j) {
+            for (int j = 0; j < kLineRegs; ++j) {
                 const double y = fma(tt, rb[j], ra[j]);
                 acc[j & 3] += y + fabs(y);
             }
@@ -595,7 +596,7 @@ struct Chain {
 #pragma unroll
             for (int b = 0; b < B; ++b) acc[b][0] = acc[b][1] = acc[b][2] = acc[b][3] = 0.0;
 #pragma unroll
-            for (int j = 0; j < NW; ++j)
+            for (int j = 0; j < kLineRegs; ++j)
 #pragma unroll
                 for (int b = 0; b < B; ++b) {
                     const double y = fma(tt[b], rb[j], ra[j]);
@@ -1189,14 +1190,8 @@ struct Chain {
     // (brent_step), reusing the batch's values for as long as the abscissae still agree.
     struct Brent { double lo, hi, x, w, v, fx, fw, fv, stp, old; };
     static constexpr double kGolden = 0.3819660112501051;  // (3 - sqrt(5)) / 2
-#ifndef PDMPFLUX_SPEC_B
-#define PDMPFLUX_SPEC_B 4
-#endif
-#ifndef PDMPFLUX_SUPER
-#define PDMPFLUX_SUPER 5
-#endif
-    static constexpr int kSuper = PDMPFLUX_SUPER;   // transposed team Brent: iterations per lane per pass
-    static constexpr int kSpecB = kRegLine ? PDMPFLUX_SPEC_B : 0;   // measured gain only where the team reduction is the latency (+4..13 %); thread-per-chain kernels are issue bound
+    static constexpr int kSuper = 5;   // transposed team Brent: iterations per lane per pass
+    static constexpr int kSpecB = kRegLine ? 4 : 0;   // measured gain only where the team reduction is the latency (+4..13 %); thread-per-chain kernels are issue bound
 
     // tolerance, midpoint and golden-section abscissa of the iteration that starts from the bracket (lo, hi) and best x
     __device__ static __forceinline__ double brent_golden(double lo, double hi, double x, double& tol, double& mid,
@@ -2502,11 +2497,9 @@ struct Chain {
 
 // One launch advances every chain by p.n_events accepted events (or just records the current state when
 // n_events == 0 and col0 names the column).  Grid = ceil(n_chains / (kBT / TEAM)).
-#ifndef PDMPFLUX_MINBLOCKS_GRID
-#define PDMPFLUX_MINBLOCKS_GRID 4
-#endif
-template <int TEAM, int SAMPLER, int POT, int PATH, int NW = 0>
-__global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH == kPathGeneric ? 1 : (PATH == kPathFastBrent ? (TEAM == 1 && SAMPLER == PDMPFLUX_ZIGZAG ? 4 : 2) : (TEAM == 32 ? 3 : PDMPFLUX_MINBLOCKS_GRID))) skeleton_kernel(const __grid_constant__ KernelParams p) {
+constexpr int kMinBlocksGrid = 4;   // grid-bound kernels of teams of 1 / 8: blocks per SM (3 measured -10 .. -13 %)
+template <int TEAM, int SAMPLER, int POT, int PATH, int NW = kLineShared>
+__global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH == kPathGeneric ? 1 : (PATH == kPathFastBrent ? (TEAM == 1 && SAMPLER == PDMPFLUX_ZIGZAG ? 4 : 2) : (TEAM == 32 ? 3 : kMinBlocksGrid))) skeleton_kernel(const __grid_constant__ KernelParams p) {
     constexpr int kBT = block_threads_rt(TEAM, SAMPLER, PATH);
     constexpr int CPB = kBT / TEAM;  // chains per block
     const int c_local = threadIdx.x / TEAM;
@@ -2534,12 +2527,12 @@ __global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH ==
     const int toff = (TEAM == 1) ? (int)threadIdx.x : c_local * p.dpad + ch.tl;  // this thread's offset in a vector
     ch.off_x = toff;
     ch.off_v = vec + toff;
-    int used = 2;
+    constexpr int kVectors = state_vectors(SAMPLER, PATH, TEAM, NW);
+    int used = kVectors;
     ch.off_a = ch.off_b = 0;
-    if constexpr (SAMPLER == PDMPFLUX_ZIGZAG && PATH == kPathFastBrent && NW <= 0 && TEAM > 1) {
+    if constexpr (kVectors == 4) {
         ch.off_a = 2 * vec + toff;
         ch.off_b = 3 * vec + toff;
-        used = 4;
     }
     {
         double* base = p.scratch_in_smem ? g_smem + (size_t)used * vec + toff

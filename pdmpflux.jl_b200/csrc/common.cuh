@@ -21,6 +21,18 @@ constexpr int kBlockThreads = 128;   // threads per block of every kernel except
 // PATH of a skeleton kernel (chain.cuh)
 enum { kPathGeneric = 0, kPathFastBrent = 1, kPathFastGrid = 2 };
 
+// Zig-Zag x Brent on a team of lanes: where the kernel keeps the line model (A_j, B_j) of the owned coordinates.  The
+// value is the NW template argument of skeleton_kernel (launch.cuh: brent_line_model picks it).
+constexpr int kLineShared = 0;       // shared-memory A / B vectors (also every kernel that has no Zig-Zag x Brent line model)
+constexpr int kLineTransposed = -1;  // transposed Brent search: every lane keeps the chain's compressed model (chain.cuh)
+constexpr int kLineRegs = 16;        // registers: at most kLineRegs owned coordinates per lane, one team reduction per rate
+
+// shared-memory state vectors of a block before the scratch / flags / moments: x, v and, where the line model keeps
+// them there, A and B
+__host__ __device__ constexpr int state_vectors(int sampler, int path, int team, int line) {
+    return sampler == PDMPFLUX_ZIGZAG && path == kPathFastBrent && team > 1 && line != kLineRegs ? 4 : 2;
+}
+
 // Thread-per-chain Zig-Zag x Brent is limited by the shared memory its chains' x and v take (16 d bytes per chain):
 // blocks of 64 threads pack the SM with four blocks (8 warps) where blocks of 128 leave room for one or two.
 // The same holds for thread-per-chain BPS / Boomerang / ForwardECMC at d ~ 100 (1.8 kB of state per chain): blocks of
@@ -97,7 +109,7 @@ struct KernelParams {
     double* scratch;
     int scratch_in_smem;
     int n_own;      // ceil(d / TEAM)
-    int brent_nw;   // Zig-Zag x Brent: the kernel variant chosen at chains_create (launch.cuh, brent_reg_nw)
+    int brent_nw;   // Zig-Zag x Brent: the line model chosen at chains_create (kLine*, launch.cuh: brent_line_model)
     int vec_elems;  // doubles per shared-memory state vector of a block (x, v, A, B, scratch each take one)
     int dpad;       // TEAM > 1: doubles reserved per chain inside a state vector (chain-contiguous layout)
     // output path

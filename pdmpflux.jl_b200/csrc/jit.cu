@@ -90,19 +90,9 @@ Nvrtc& nvrtc() {
     return n;
 }
 
-// -D values the library itself was built with: the run-time kernels must be the same code as the built-in ones
+// the host's KernelParams size: jit_source.cuh checks that the run-time kernels see the same layout
 std::string defines() {
-    std::string s = "#define PDMPFLUX_HOST_KERNEL_PARAMS_BYTES " + std::to_string(sizeof(KernelParams)) + "\n";
-#ifdef PDMPFLUX_MINBLOCKS_GRID
-    s += "#define PDMPFLUX_MINBLOCKS_GRID " PDMPFLUX_STR(PDMPFLUX_MINBLOCKS_GRID) "\n";
-#endif
-#ifdef PDMPFLUX_SPEC_B
-    s += "#define PDMPFLUX_SPEC_B " PDMPFLUX_STR(PDMPFLUX_SPEC_B) "\n";
-#endif
-#ifdef PDMPFLUX_SUPER
-    s += "#define PDMPFLUX_SUPER " PDMPFLUX_STR(PDMPFLUX_SUPER) "\n";
-#endif
-    return s;
+    return "#define PDMPFLUX_HOST_KERNEL_PARAMS_BYTES " + std::to_string(sizeof(KernelParams)) + "\n";
 }
 
 struct Entry {

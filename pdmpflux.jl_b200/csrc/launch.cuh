@@ -1,34 +1,35 @@
 // Host-side dispatch from (team width, potential kind) to a kernel instantiation.
 #pragma once
-#include <cstdlib>
-
 #include "chain.cuh"
 
 namespace pdmpflux {
 
-// Zig-Zag + Brent on a team of lanes: which line model the kernel keeps (the NW template argument).
-//   -1  transposed Brent: teams of 8 with at most 8 owned coordinates per lane (d <= 64) -- every lane keeps the chain's
-//       compressed model and takes its own iterations of the search (chain.cuh, build_bound_brent)
-//   8 / 16  register-resident (A_j, B_j) of the owned coordinates, team reduction per rate evaluation
-//   0   the shared-memory A/B arrays
-// Mirrors the instantiations below; api.cu sizes the shared memory with it.  PDMPFLUX_TSPEC=0 switches the transposed
-// search off (the tests compare the two).
-inline int brent_reg_nw(int sampler, int path, int team, int n_own) {
-    if (sampler != PDMPFLUX_ZIGZAG || path != kPathFastBrent) return 0;
-    if (team != 4 && team != 8) return 0;
-    if (team == 8 && n_own <= 8) {
-        const char* e = std::getenv("PDMPFLUX_TSPEC");
-        if (!e || std::atoi(e) != 0) return -1;
-    }
-    return n_own <= 8 ? 8 : (n_own <= 16 ? 16 : 0);
+// Zig-Zag + Brent on a team of lanes: which line model the kernel keeps (the NW template argument, common.cuh).
+//   kLineTransposed  teams of 8 with at most 8 owned coordinates per lane (d <= 64) -- every lane keeps the chain's
+//                    compressed model and takes its own iterations of the search (chain.cuh, build_bound_brent)
+//   kLineRegs        teams of 8 with at most 16 owned coordinates per lane (d <= 128): register-resident (A_j, B_j),
+//                    team reduction per rate evaluation
+//   kLineShared      the shared-memory A/B arrays (every other team and sampler)
+// launch_for_pot instantiates exactly these; api.cu sizes the shared memory with it.
+inline int brent_line_model(int sampler, int path, int team, int n_own) {
+    if (sampler != PDMPFLUX_ZIGZAG || path != kPathFastBrent || team != 8) return kLineShared;
+    if (n_own <= 8) return kLineTransposed;
+    return n_own <= kLineRegs ? kLineRegs : kLineShared;
 }
 
-template <int TEAM, int SAMPLER, int POT, int PATH, int NW = 0>
+// whether a sampler has a fast path (kPathFastBrent / kPathFastGrid) for a potential with these traits
+constexpr bool has_fast_path(int sampler, bool affine, int n_special) {
+    return affine && sampler != PDMPFLUX_STICKY_ZIGZAG   // masked velocities: per-node evaluation only
+           && sampler != PDMPFLUX_SPEEDUP_ZIGZAG         // nonlinear flow: no affine line model
+           && !(sampler == PDMPFLUX_BOOMERANG && n_special > 0);
+}
+template <int POT>
+constexpr bool has_fast_path(int sampler) { return has_fast_path(sampler, Pot<POT>::kAffine, Pot<POT>::kSpecial); }
+
+template <int TEAM, int SAMPLER, int POT, int PATH, int NW = kLineShared>
 cudaError_t launch_one(const KernelParams& p, unsigned grid, size_t smem, cudaStream_t stream) {
-    // combinations without a fast path fall back to the generic kernel (same results, more passes)
-    constexpr bool ok = PATH == kPathGeneric ||
-                        (SAMPLER != PDMPFLUX_STICKY_ZIGZAG && SAMPLER != PDMPFLUX_SPEEDUP_ZIGZAG && Pot<POT>::kAffine &&
-                         !(SAMPLER == PDMPFLUX_BOOMERANG && Pot<POT>::kSpecial > 0));
+    // no fast-path kernel is built where select_path never picks one
+    constexpr bool ok = PATH == kPathGeneric || has_fast_path<POT>(SAMPLER);
     if constexpr (!ok) return cudaErrorInvalidValue;
     else {
         auto kern = skeleton_kernel<TEAM, SAMPLER, POT, PATH, NW>;
@@ -43,29 +44,18 @@ cudaError_t launch_one(const KernelParams& p, unsigned grid, size_t smem, cudaSt
 
 template <int TEAM, int SAMPLER, int POT>
 cudaError_t launch_for_pot(int path, const KernelParams& p, unsigned grid, size_t smem, cudaStream_t stream) {
-    if constexpr (TEAM == 4) {  // only built for the register-resident Zig-Zag x Brent kernels
-        if constexpr (SAMPLER == PDMPFLUX_ZIGZAG && Pot<POT>::kAffine) {
+    switch (path) {
+    case kPathGeneric: return launch_one<TEAM, SAMPLER, POT, kPathGeneric>(p, grid, smem, stream);
+    case kPathFastBrent:
+        if constexpr (TEAM == 8 && SAMPLER == PDMPFLUX_ZIGZAG && Pot<POT>::kAffine) {
             switch (p.brent_nw) {
-            case 8: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, 8>(p, grid, smem, stream);
-            case 16: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, 16>(p, grid, smem, stream);
+            case kLineTransposed: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, kLineTransposed>(p, grid, smem, stream);
+            case kLineRegs: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, kLineRegs>(p, grid, smem, stream);
             }
         }
-        return cudaErrorInvalidValue;
-    } else {
-        switch (path) {
-        case kPathGeneric: return launch_one<TEAM, SAMPLER, POT, kPathGeneric>(p, grid, smem, stream);
-        case kPathFastBrent:
-            if constexpr (TEAM == 8 && SAMPLER == PDMPFLUX_ZIGZAG && Pot<POT>::kAffine) {
-                switch (p.brent_nw) {
-                case -1: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, -1>(p, grid, smem, stream);
-                case 8: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, 8>(p, grid, smem, stream);
-                case 16: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, 16>(p, grid, smem, stream);
-                }
-            }
-            return launch_one<TEAM, SAMPLER, POT, kPathFastBrent>(p, grid, smem, stream);
-        case kPathFastGrid: return launch_one<TEAM, SAMPLER, POT, kPathFastGrid>(p, grid, smem, stream);
-        default: return cudaErrorInvalidValue;
-        }
+        return launch_one<TEAM, SAMPLER, POT, kPathFastBrent>(p, grid, smem, stream);
+    case kPathFastGrid: return launch_one<TEAM, SAMPLER, POT, kPathFastGrid>(p, grid, smem, stream);
+    default: return cudaErrorInvalidValue;
     }
 }
 
@@ -87,25 +77,23 @@ cudaError_t launch_for_sampler(int team, int pot, int path, const KernelParams& 
                                cudaStream_t stream) {
     switch (team) {
     case 1: return launch_for_team<1, SAMPLER>(pot, path, p, grid, smem, stream);
-    case 4:
-        if constexpr (SAMPLER == PDMPFLUX_ZIGZAG) return launch_for_team<4, SAMPLER>(pot, path, p, grid, smem, stream);
-        else return cudaErrorInvalidValue;
-#ifdef PDMPFLUX_EXTRA_TEAM
-    case PDMPFLUX_EXTRA_TEAM: return launch_for_team<PDMPFLUX_EXTRA_TEAM, SAMPLER>(pot, path, p, grid, smem, stream);
-#endif
     case 8: return launch_for_team<8, SAMPLER>(pot, path, p, grid, smem, stream);
     case 32: return launch_for_team<32, SAMPLER>(pot, path, p, grid, smem, stream);
     default: return cudaErrorInvalidValue;
     }
 }
 
-// which path a (sampler, potential, config) combination runs on; mirrors the `ok` condition of launch_one
+// which path a (sampler, potential, config) combination runs on: a fast path exactly where launch_one builds one
 inline int select_path(int sampler, int pot, int grid_size, int vectorized, int deriv_mode) {
-    const bool affine = pot == PDMPFLUX_GAUSS_STD || pot == PDMPFLUX_GAUSS_DIAG || pot == PDMPFLUX_GAUSS_EQUICORR ||
-                        pot == PDMPFLUX_BANANA;
-    if (!affine || (sampler == PDMPFLUX_BOOMERANG && pot == PDMPFLUX_BANANA)) return kPathGeneric;
-    if (sampler == PDMPFLUX_STICKY_ZIGZAG) return kPathGeneric;  // masked velocities: per-node evaluation only
-    if (sampler == PDMPFLUX_SPEEDUP_ZIGZAG) return kPathGeneric; // nonlinear flow: no affine line model
+    bool fast = false;
+    switch (pot) {
+    case PDMPFLUX_GAUSS_STD: fast = has_fast_path<PDMPFLUX_GAUSS_STD>(sampler); break;
+    case PDMPFLUX_GAUSS_DIAG: fast = has_fast_path<PDMPFLUX_GAUSS_DIAG>(sampler); break;
+    case PDMPFLUX_GAUSS_EQUICORR: fast = has_fast_path<PDMPFLUX_GAUSS_EQUICORR>(sampler); break;
+    case PDMPFLUX_BANANA: fast = has_fast_path<PDMPFLUX_BANANA>(sampler); break;
+    case PDMPFLUX_BANANA_README_SCALAR: fast = has_fast_path<PDMPFLUX_BANANA_README_SCALAR>(sampler); break;
+    }
+    if (!fast) return kPathGeneric;
     if (grid_size == 0) return kPathFastBrent;
     if (sampler == PDMPFLUX_ZIGZAG) {
         // vectorised bound with analytic derivatives only: with finite differences the reference's cell maximum

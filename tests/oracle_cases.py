@@ -25,6 +25,12 @@ CASES = [
     # monotone on the bracket and Brent's search changes direction, fails golden steps and ends at either end -- every
     # branch of the speculative search is exercised.  (Not a distribution; the short run stays finite.)
     ("zz_saddle20_brent", ZIGZAG, GAUSS_DIAG, "mixed_sign", 20, dict(grid_size=0, tmax=0.5), 250),
+    # 64 < d <= 128: teams of 8 keep the line model in registers and evaluate four predicted abscissae per batch.  The
+    # banana's special coordinates, fixed horizons, a saddle (the batches' replay branches) and the top of the range.
+    ("zz_banana100_brent", ZIGZAG, BANANA, None, 100, dict(grid_size=0), 300),
+    ("zz_gauss80_brent_nonadaptive", ZIGZAG, GAUSS_STD, None, 80, dict(grid_size=0, adaptive=False, tmax=0.7), 300),
+    ("zz_saddle96_brent", ZIGZAG, GAUSS_DIAG, "mixed_sign", 96, dict(grid_size=0, tmax=0.5), 250),
+    ("zz_diag128_brent", ZIGZAG, GAUSS_DIAG, "linspace", 128, dict(grid_size=0), 300),
     ("zz_banana5_grid_fd", ZIGZAG, BANANA, None, 5, dict(grid_size=8, deriv_mode=1), 1000),
     ("zz_banana40_jvp", ZIGZAG, BANANA, None, 40, dict(grid_size=6), 800),
     ("zz_readme_scalar", ZIGZAG, BANANA_README, None, 6, dict(grid_size=0), 7),

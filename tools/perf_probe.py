@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Device-resident throughput of the BASELINE configurations (kernel time by CUDA events; not a bench line).
 
-usage: tools/perf_probe.py SPEC [SPEC ...]     SPEC = config[:chains[:events[:team]]]   e.g.  c2:4096:1000:4  c5f
+usage: tools/perf_probe.py SPEC [SPEC ...]     SPEC = config[:chains[:events[:team]]]   e.g.  c2:4096:1000:8  c5f
 Each spec runs in a fresh subprocess-free loop: warm-up launch, then best of 3 timed launches; full PDMPHistory stored.
 """
 import os
