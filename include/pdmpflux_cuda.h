@@ -173,7 +173,27 @@ int pdmpflux_potential_destroy(pdmpflux_potential_t pot);
  * pp.vec is a device copy of params[0 .. n_params-1] and pp.n = n_params.  The gradient may depend on the whole vector
  * only through the K functionals.  The source is compiled with NVRTC (bound at run time; ERR_UNSUPPORTED without it):
  * a contract check here (ERR_COMPILE with the log, lines numbered as `user_potential(<line>)`), the kernels when a
- * sampler is created.  Every sampler kind runs it on the generic kernel; pdmpflux_rv_diagnostic does not (no U value). */
+ * sampler is created.  pdmpflux_rv_diagnostic does not run it (no U value).
+ *
+ * Optional members declare the line model of the built-in plugins and put the potential on the fast-path kernels
+ * (Zig-Zag x Brent, the Zig-Zag affine-cell grid bound, the BPS / ForwardECMC line sums); without them every sampler
+ * runs the generic kernel:
+ *
+ *   static constexpr bool affine = true;  for every i >= special the Hessian is constant along the flow line:
+ *                                         g_i(x + t v) = g_i(x) + t (H v)_i exactly, (H v)_i being the hd of eval
+ *   static constexpr int special = 2;     0 <= special <= K, needs affine: L_k(x) = x_k for k < special (accum puts
+ *                                         x_k, and nothing else, into acc[k]); these coordinates' rates are evaluated
+ *                                         per time from the functionals
+ *   __device__ static void eval_local(const pdmpflux::PotParams&, int i, double xi, double di, double& gl, double& hl);
+ *   __device__ static void line_corr(const pdmpflux::PotParams&, const double* Lx, const double* Ld, double& ca, double& cb);
+ *                                         both or neither, need affine and special = 0: gl, hl are the parts of g_i and
+ *                                         (H d)_i that do not involve the functionals; ca = sum_i (g_i - gl_i) d_i and
+ *                                         cb = sum_i ((H d)_i - hl_i) d_i, from the functionals alone
+ *
+ * A declaration that breaks one of these rules is an ERR_COMPILE naming the member.  Whether the potential really has
+ * the declared structure cannot be checked, just as the linearity of accum cannot: a wrong declaration samples the
+ * wrong target.  Boomerang keeps the generic kernel for a source (its fast path needs grad U(0) = 0, which affine does
+ * not promise). */
 int pdmpflux_potential_create_source(int dim, const char* source, const double* params, int64_t n_params,
                                      pdmpflux_potential_t* out);
 

@@ -64,6 +64,10 @@ LogReg(X::AbstractMatrix, y::AbstractVector, sigma0::Real) =
 A potential written in CUDA C++: `source` defines `struct UserPotential` (K linear functionals, `accum`, `grad`,
 `eval`; the contract is stated in include/pdmpflux_cuda.h above `pdmpflux_potential_create_source`) and `params` are
 `pp.vec[0 .. pp.n-1]` on the device.  Compiled at run time with NVRTC when the sampler is constructed.
+
+The optional members `affine`, `special`, `eval_local` and `line_corr` declare the potential's line model (same header)
+and put it on the fast-path kernels of Zig-Zag, BPS and ForwardECMC; without them it runs the generic kernel.  The
+library cannot check that the potential has the declared structure: a wrong declaration samples the wrong target.
 """
 CudaPotential(source::AbstractString, params::AbstractVector=Float64[]) =
     CuPotential(Int32(6), collect(Float64, params), String(source))

@@ -71,6 +71,7 @@ struct pdmpflux_potential_s {
     PotParams pp{};
     DevBuf params;
     std::string source;  // PDMPFLUX_SOURCE: the user's CUDA text (jit.cu)
+    SourceTraits traits; // PDMPFLUX_SOURCE: the line model it declares (read by the contract check)
 };
 
 // Device slabs of the host-buffer pipeline, cached in the sampler handle so that repeated sample_skeleton calls do
@@ -179,6 +180,32 @@ int widen_team(int team, int sampler, int path, int d) {
     return team;
 }
 
+// the line-model traits select_path sees for this sampler: a built-in kind's Pot<> traits, a source's declared ones.
+// Boomerang keeps a source on the generic kernel: its fast path takes <grad U(x), x> as <P x, x>, which holds only when
+// grad U(0) = 0 -- true of every built-in, not promised by an affine declaration (a Gaussian with a non-zero mean).
+LineTraits line_traits(int sampler, const pdmpflux_potential_s* pot) {
+    if (pot->kind != PDMPFLUX_SOURCE) return builtin_line_traits(pot->kind);
+    if (sampler == PDMPFLUX_BOOMERANG) return {};
+    return {pot->traits.affine, pot->traits.special};
+}
+
+// The kernel variant that n_chains chains of a sampler run: path, team width and Zig-Zag x Brent line model.
+// with_env: honour PDMPFLUX_FORCE_GENERIC and PDMPFLUX_TEAM (pdmpflux_chains_create); without: the default policy,
+// which is what sampler creation compiles ahead for a source potential.
+struct Variant { int path, team, n_own, nw; };
+Variant chain_variant(int kind, int dim, const pdmpflux_config& cfg, const pdmpflux_potential_s* pot, int64_t n_chains,
+                      bool with_env) {
+    Variant v{};
+    v.path = select_path(kind, line_traits(kind, pot), cfg.grid_size, cfg.vectorized_bound, cfg.deriv_mode);
+    if (const char* e = with_env ? std::getenv("PDMPFLUX_FORCE_GENERIC") : nullptr) { if (std::atoi(e)) v.path = kPathGeneric; }
+    const bool zz_brent_fast = kind == PDMPFLUX_ZIGZAG && v.path == kPathFastBrent && pot->kind != PDMPFLUX_LOGREG;
+    const int team = with_env ? pick_team(dim, n_chains, zz_brent_fast) : default_team(dim, n_chains, zz_brent_fast);
+    v.team = widen_team(team, kind, v.path, dim);
+    v.n_own = (dim + v.team - 1) / v.team;
+    v.nw = brent_line_model(kind, v.path, v.team, v.n_own);
+    return v;
+}
+
 // `rows`: optional separate placement of the X / V rows (host pipeline: rows go through narrow double-buffered
 // slabs while the scalar columns accumulate in full-length device buffers)
 struct RowsView { double *X, *V; int64_t ld, col0; };
@@ -246,7 +273,7 @@ int launch(pdmpflux_chains_s* ch, int64_t n_events, const pdmpflux_history* h, i
     const size_t smem_launch = ch->smem + (ch->moments ? 2 * (size_t)ch->vec_elems * sizeof(double) : 0);
     if (smem_launch > 227 * 1024) return fail(PDMPFLUX_ERR_UNSUPPORTED, "fused moments: shared memory exhausted for this dimension");
     if (s->pot->kind == PDMPFLUX_SOURCE) {
-        const int rc = jit_launch(s->pot->source, s->kind, ch->team, p, ch->grid, smem_launch, stream);
+        const int rc = jit_launch(s->pot->source, s->kind, ch->team, ch->path, ch->brent_nw, p, ch->grid, smem_launch, stream);
         if (rc != PDMPFLUX_OK) return rc;
         e = cudaSuccess;
     } else if (s->pot->kind == PDMPFLUX_LOGREG) {
@@ -542,7 +569,7 @@ int pdmpflux_potential_create_source(int dim, const char* source, const double* 
     auto pot = std::make_unique<pdmpflux_potential_s>();
     pot->kind = PDMPFLUX_SOURCE; pot->dim = dim; pot->source = source;
     // the contract check runs before any CUDA call: bad source fails here, with or without a device
-    const int rc = jit_check_source(pot->source);
+    const int rc = jit_check_source(pot->source, &pot->traits);
     if (rc != PDMPFLUX_OK) return rc;
     if (n_params > 0) {
         if (pot->params.alloc(sizeof(double) * (size_t)n_params) != cudaSuccess ||
@@ -586,18 +613,20 @@ static int sampler_create_impl(int kind, int dim, pdmpflux_potential_t pot, cons
     if (kind == PDMPFLUX_FECMC && dim < 2)
         return fail(PDMPFLUX_ERR_ARGUMENT, "The dimension must be at least 2 to use the ForwardEventChain. Got dimension " + std::to_string(dim));
     if (!(cfg->tmax >= 0.0) || !std::isfinite(cfg->tmax)) return fail(PDMPFLUX_ERR_ARGUMENT, "tmax must be finite and >= 0");
+    pdmpflux_config ncfg = *cfg;
+    normalise_config(kind, dim, ncfg);
     if (pot->kind == PDMPFLUX_SOURCE) {
-        // compile every team width the default policy can pick for this (kind, dim) -- the kernel is the generic one
-        // whatever the config -- before any CUDA call, so that source errors surface here even without a device
+        // compile every kernel variant the default policy can pick for this sampler (the team widths chosen at one
+        // chain and at any number of chains) before any CUDA call, so that source errors surface here even without a
+        // device
         for (int64_t n_chains : {int64_t(1), INT64_MAX}) {
-            const int team = widen_team(default_team(dim, n_chains, false), kind, kPathGeneric, dim);
-            const int rc = jit_prepare(pot->source, kind, team);
+            const Variant v = chain_variant(kind, dim, ncfg, pot, n_chains, false);
+            const int rc = jit_prepare(pot->source, kind, v.team, v.path, v.nw);
             if (rc != PDMPFLUX_OK) return rc;
         }
     }
     auto s = new pdmpflux_sampler_s();
-    s->kind = kind; s->dim = dim; s->cfg = *cfg; s->pot = pot;
-    normalise_config(kind, dim, s->cfg);
+    s->kind = kind; s->dim = dim; s->cfg = ncfg; s->pot = pot;
     if (kind == PDMPFLUX_STICKY_ZIGZAG) {
         for (int i = 0; i < dim; ++i)
             if (!(kappa[i] >= 0.0) || !std::isfinite(kappa[i])) { delete s; return fail(PDMPFLUX_ERR_ARGUMENT, "kappa must be finite and non-negative"); }
@@ -648,15 +677,12 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
     ch->s = s; ch->n_chains = n_chains; ch->chain_offset = chain_offset; ch->seed = seed;
     const int d = s->dim;
     const bool logreg = s->pot->kind == PDMPFLUX_LOGREG;
-    ch->path = select_path(s->kind, s->pot->kind, s->cfg.grid_size, s->cfg.vectorized_bound, s->cfg.deriv_mode);
-    if (const char* e = std::getenv("PDMPFLUX_FORCE_GENERIC")) { if (std::atoi(e)) ch->path = kPathGeneric; }
-    const bool zz_brent_fast = s->kind == PDMPFLUX_ZIGZAG && ch->path == kPathFastBrent && !logreg;
-    ch->team = widen_team(pick_team(d, n_chains, zz_brent_fast), s->kind, ch->path, d);
-    if (s->pot->kind == PDMPFLUX_SOURCE) {  // a width sampler_create did not compile (PDMPFLUX_TEAM): compile it now
-        const int rc = jit_prepare(s->pot->source, s->kind, ch->team);
+    const Variant var = chain_variant(s->kind, d, s->cfg, s->pot, n_chains, true);
+    ch->path = var.path; ch->team = var.team; ch->n_own = var.n_own; ch->brent_nw = var.nw;
+    if (s->pot->kind == PDMPFLUX_SOURCE) {  // a variant sampler_create did not compile (PDMPFLUX_TEAM / _FORCE_GENERIC)
+        const int rc = jit_prepare(s->pot->source, s->kind, ch->team, ch->path, ch->brent_nw);
         if (rc != PDMPFLUX_OK) return rc;
     }
-    ch->n_own = (d + ch->team - 1) / ch->team;
     const int bt = block_threads_rt(ch->team, s->kind, ch->path);   // threads per block of the kernel that will run
     const int cpb = bt / ch->team;
     ch->grid = (unsigned)((n_chains + cpb - 1) / cpb);
@@ -668,7 +694,6 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
         ch->vec_elems = cpb * ch->dpad;
     }
     const size_t vec_bytes = (size_t)ch->vec_elems * sizeof(double);
-    ch->brent_nw = brent_line_model(s->kind, ch->path, ch->team, ch->n_own);
     const size_t nvec = state_vectors(s->kind, ch->path, ch->team, ch->brent_nw);
     ch->smem = (nvec + (s->kind == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) * vec_bytes;
     const size_t list_slack = ch->brent_nw == kLineTransposed ? 16 * sizeof(double) : 0;   // transposed Brent: unconditional reads of the 12-slot list

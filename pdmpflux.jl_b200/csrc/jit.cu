@@ -1,5 +1,6 @@
 // Source potentials: user-written CUDA (jit_source.cuh states the contract) compiled at run time with NVRTC into the
-// generic thinning kernel of chain.cuh, then loaded and launched like the built-in instantiations.
+// thinning kernels of chain.cuh -- the generic one, or the fast paths for a source that declares a line model -- then
+// loaded and launched like the built-in instantiations.
 //
 // NVRTC is bound at run time (dlopen), so the library keeps no link-time dependency on it.  The toolkit the library was
 // built with is tried first: the process may already hold another libnvrtc.so.12 (PyTorch bundles one), and a
@@ -8,7 +9,7 @@
 // nothing but libnvrtc.
 //
 // Compiled cubins live in one process-wide cache keyed by everything that determines them (source, headers, NVRTC
-// version, sampler kind, team width, defines) -- not by the potential handle, which the Python binding creates afresh
+// version, sampler kind, team width, path, line model, defines) -- not by the potential handle, which the Python binding creates afresh
 // for every sampler.  Parameters are run-time data and never part of the key.
 #include <dlfcn.h>
 
@@ -97,6 +98,7 @@ std::string defines() {
 
 struct Entry {
     std::string cubin, lowered;
+    SourceTraits traits;               // the contract check: what the source declares
     cudaLibrary_t library = nullptr;   // loaded on first launch (context independent: serves every device)
     cudaKernel_t kernel = nullptr;
 };
@@ -124,7 +126,11 @@ uint64_t headers_hash() {
     return h;
 }
 
-// kind < 0: the contract-check program; otherwise the generic skeleton kernel for (kind, team)
+// kind < 0: the contract-check program; otherwise the skeleton kernels.  The check also instantiates an empty kernel
+// whose template arguments are the traits of Pot<PDMPFLUX_SOURCE>: its lowered (mangled) name carries them back to the
+// host without a CUDA call.
+const char kTraitsName[] = "&pdmpflux_traits<pdmpflux::Pot<PDMPFLUX_SOURCE>::K, pdmpflux::Pot<PDMPFLUX_SOURCE>::kAffine, "
+                           "pdmpflux::Pot<PDMPFLUX_SOURCE>::kSpecial, pdmpflux::Pot<PDMPFLUX_SOURCE>::kSplit>";
 std::string program_text(const std::string& source, int kind) {
     std::string s = defines();
     s += "#include \"potentials.cuh\"\n#line 1 \"user_potential\"\n";
@@ -137,23 +143,51 @@ std::string program_text(const std::string& source, int kind) {
              "    P::accum(pp, threadIdx.x, out[0], acc);\n"
              "    P::eval(pp, threadIdx.x, out[0], out[1], acc, Ld, g, hd);\n"
              "    out[2] = P::grad(pp, threadIdx.x, out[0], acc) + g + hd;\n"
-             "}\n";
+             "}\n"
+             "template <int K, bool Affine, int Special, bool Split> __global__ void pdmpflux_traits() {}\n";
     else s += "#include \"chain.cuh\"\n";
     return s;
 }
 
-std::string kernel_name(int kind, int team) {
+std::string kernel_name(int kind, int team, int path, int nw) {
     return "pdmpflux::skeleton_kernel<" + std::to_string(team) + ", " + std::to_string(kind) + ", " +
-           std::to_string((int)PDMPFLUX_SOURCE) + ", " + std::to_string((int)kPathGeneric) + ", 0>";
+           std::to_string((int)PDMPFLUX_SOURCE) + ", " + std::to_string(path) + ", " + std::to_string(nw) + ">";
 }
 
-// Compiles (or finds) the program for (source, kind, team).  Caller holds the cache mutex.
-int get_entry(const std::string& source, int kind, int team, Entry** out) {
+// Reads the template arguments of pdmpflux_traits<K, kAffine, kSpecial, kSplit> out of its Itanium-mangled name,
+// e.g. _Z15pdmpflux_traitsILi2ELb1ELi2ELb0EEvv: integer literals "L<type><value>E", a negative value as "n<digits>".
+bool parse_traits(const std::string& lowered, SourceTraits& t) {
+    const size_t open = lowered.find("pdmpflux_traitsI");
+    if (open == std::string::npos) return false;
+    size_t pos = open + sizeof("pdmpflux_traitsI") - 1;
+    const char types[4] = {'i', 'b', 'i', 'b'};
+    long v[4];
+    for (int k = 0; k < 4; ++k) {
+        if (pos + 2 >= lowered.size() || lowered[pos] != 'L' || lowered[pos + 1] != types[k]) return false;
+        pos += 2;
+        const bool neg = lowered[pos] == 'n';
+        if (neg) ++pos;
+        size_t digits = 0;
+        long x = 0;
+        while (pos < lowered.size() && lowered[pos] >= '0' && lowered[pos] <= '9' && digits < 9) {
+            x = 10 * x + (lowered[pos++] - '0');
+            ++digits;
+        }
+        if (digits == 0 || pos >= lowered.size() || lowered[pos++] != 'E') return false;
+        v[k] = neg ? -x : x;
+    }
+    if (pos >= lowered.size() || lowered[pos] != 'E') return false;
+    t.K = (int)v[0]; t.affine = v[1] != 0; t.special = (int)v[2]; t.split = v[3] != 0;
+    return true;
+}
+
+// Compiles (or finds) the program for (source, kind, team, path, nw).  Caller holds the cache mutex.
+int get_entry(const std::string& source, int kind, int team, int path, int nw, Entry** out) {
     Nvrtc& nv = nvrtc();
     if (!nv.lib) return pdmpflux_fail_(PDMPFLUX_ERR_UNSUPPORTED, nv.why);
     const std::string text = program_text(source, kind);
     const std::string key = nv.version + '\0' + std::to_string(headers_hash()) + '\0' + std::to_string(kind) + '\0' +
-                            std::to_string(team) + '\0' + text;
+                            std::to_string(team) + '\0' + std::to_string(path) + '\0' + std::to_string(nw) + '\0' + text;
     Cache& c = cache();
     auto it = c.entries.find(key);
     if (it != c.entries.end()) { *out = it->second.get(); return PDMPFLUX_OK; }
@@ -165,8 +199,8 @@ int get_entry(const std::string& source, int kind, int team, Entry** out) {
     int r = nv.CreateProgram(&prog, text.c_str(), "pdmpflux_source_potential.cu", kNumHeaders, texts, names);
     if (r != 0) return pdmpflux_fail_(PDMPFLUX_ERR_COMPILE, std::string("nvrtcCreateProgram: ") + nv.GetErrorString(r));
     struct Guard { Nvrtc& nv; Nvrtc::Prog* p; ~Guard() { nv.DestroyProgram(p); } } guard{nv, &prog};
-    const std::string name = kind < 0 ? std::string() : kernel_name(kind, team);
-    if (kind >= 0 && (r = nv.AddNameExpression(prog, name.c_str())) != 0)
+    const std::string name = kind < 0 ? std::string(kTraitsName) : kernel_name(kind, team, path, nw);
+    if ((r = nv.AddNameExpression(prog, name.c_str())) != 0)
         return pdmpflux_fail_(PDMPFLUX_ERR_COMPILE, std::string("nvrtcAddNameExpression: ") + nv.GetErrorString(r));
     // nvcc's defaults (what the built-in kernels are compiled with), stated explicitly
     const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "--fmad=true", "--ftz=false", "--prec-div=true",
@@ -186,7 +220,12 @@ int get_entry(const std::string& source, int kind, int team, Entry** out) {
                                                         (kind < 0 ? std::string("contract check") : name) + "):\n" + log);
     }
     auto e = std::make_unique<Entry>();
-    if (kind >= 0) {
+    if (kind < 0) {
+        const char* lowered = nullptr;
+        if (nv.GetLoweredName(prog, name.c_str(), &lowered) != 0 || !lowered || !parse_traits(lowered, e->traits))
+            return pdmpflux_fail_(PDMPFLUX_ERR_COMPILE, "NVRTC " + nv.version + ": cannot read the potential's traits from the "
+                                                        "lowered name '" + std::string(lowered ? lowered : "(none)") + "'");
+    } else {
         size_t n = 0;
         const char* lowered = nullptr;
         if (nv.GetCUBINSize(prog, &n) != 0 || n == 0 || nv.GetLoweredName(prog, name.c_str(), &lowered) != 0 || !lowered)
@@ -202,24 +241,26 @@ int get_entry(const std::string& source, int kind, int team, Entry** out) {
 
 }  // namespace
 
-int jit_check_source(const std::string& source) {
+int jit_check_source(const std::string& source, SourceTraits* traits) {
     std::lock_guard<std::mutex> lk(cache().mu);
     Entry* e = nullptr;
-    return get_entry(source, -1, 0, &e);
+    const int rc = get_entry(source, -1, 0, kPathGeneric, kLineShared, &e);
+    if (rc == PDMPFLUX_OK && traits) *traits = e->traits;
+    return rc;
 }
 
-int jit_prepare(const std::string& source, int sampler_kind, int team) {
+int jit_prepare(const std::string& source, int sampler_kind, int team, int path, int nw) {
     std::lock_guard<std::mutex> lk(cache().mu);
     Entry* e = nullptr;
-    return get_entry(source, sampler_kind, team, &e);
+    return get_entry(source, sampler_kind, team, path, nw, &e);
 }
 
-int jit_launch(const std::string& source, int sampler_kind, int team, const KernelParams& p, unsigned grid, size_t smem,
-               cudaStream_t stream) {
+int jit_launch(const std::string& source, int sampler_kind, int team, int path, int nw, const KernelParams& p,
+               unsigned grid, size_t smem, cudaStream_t stream) {
     Entry* e = nullptr;
     {
         std::lock_guard<std::mutex> lk(cache().mu);
-        int rc = get_entry(source, sampler_kind, team, &e);
+        int rc = get_entry(source, sampler_kind, team, path, nw, &e);
         if (rc != PDMPFLUX_OK) return rc;
         if (!e->kernel) {
             cudaError_t ce = cudaLibraryLoadData(&e->library, e->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
@@ -238,7 +279,7 @@ int jit_launch(const std::string& source, int sampler_kind, int team, const Kern
     }
     void* args[] = {const_cast<KernelParams*>(&p)};
     const cudaError_t ce = cudaLaunchKernel(reinterpret_cast<const void*>(e->kernel), dim3(grid),
-                                            dim3(block_threads_rt(team, sampler_kind, kPathGeneric)), args, smem, stream);
+                                            dim3(block_threads_rt(team, sampler_kind, path)), args, smem, stream);
     if (ce != cudaSuccess) return pdmpflux_fail_(PDMPFLUX_ERR_CUDA, std::string("skeleton kernel launch (source potential): ") + cudaGetErrorString(ce));
     return PDMPFLUX_OK;
 }

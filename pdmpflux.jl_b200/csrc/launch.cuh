@@ -83,17 +83,23 @@ cudaError_t launch_for_sampler(int team, int pot, int path, const KernelParams& 
     }
 }
 
-// which path a (sampler, potential, config) combination runs on: a fast path exactly where launch_one builds one
-inline int select_path(int sampler, int pot, int grid_size, int vectorized, int deriv_mode) {
-    bool fast = false;
+// the line-model traits (kAffine, kSpecial) of a built-in potential kind (potentials.cuh); none for the others
+struct LineTraits { bool affine = false; int special = 0; };
+inline LineTraits builtin_line_traits(int pot) {
     switch (pot) {
-    case PDMPFLUX_GAUSS_STD: fast = has_fast_path<PDMPFLUX_GAUSS_STD>(sampler); break;
-    case PDMPFLUX_GAUSS_DIAG: fast = has_fast_path<PDMPFLUX_GAUSS_DIAG>(sampler); break;
-    case PDMPFLUX_GAUSS_EQUICORR: fast = has_fast_path<PDMPFLUX_GAUSS_EQUICORR>(sampler); break;
-    case PDMPFLUX_BANANA: fast = has_fast_path<PDMPFLUX_BANANA>(sampler); break;
-    case PDMPFLUX_BANANA_README_SCALAR: fast = has_fast_path<PDMPFLUX_BANANA_README_SCALAR>(sampler); break;
+    case PDMPFLUX_GAUSS_STD: return {Pot<PDMPFLUX_GAUSS_STD>::kAffine, Pot<PDMPFLUX_GAUSS_STD>::kSpecial};
+    case PDMPFLUX_GAUSS_DIAG: return {Pot<PDMPFLUX_GAUSS_DIAG>::kAffine, Pot<PDMPFLUX_GAUSS_DIAG>::kSpecial};
+    case PDMPFLUX_GAUSS_EQUICORR: return {Pot<PDMPFLUX_GAUSS_EQUICORR>::kAffine, Pot<PDMPFLUX_GAUSS_EQUICORR>::kSpecial};
+    case PDMPFLUX_BANANA: return {Pot<PDMPFLUX_BANANA>::kAffine, Pot<PDMPFLUX_BANANA>::kSpecial};
+    case PDMPFLUX_BANANA_README_SCALAR:
+        return {Pot<PDMPFLUX_BANANA_README_SCALAR>::kAffine, Pot<PDMPFLUX_BANANA_README_SCALAR>::kSpecial};
+    default: return {};
     }
-    if (!fast) return kPathGeneric;
+}
+
+// which path a (sampler, potential traits, config) combination runs on: a fast path exactly where launch_one builds one
+inline int select_path(int sampler, LineTraits pt, int grid_size, int vectorized, int deriv_mode) {
+    if (!has_fast_path(sampler, pt.affine, pt.special)) return kPathGeneric;
     if (grid_size == 0) return kPathFastBrent;
     if (sampler == PDMPFLUX_ZIGZAG) {
         // vectorised bound with analytic derivatives only: with finite differences the reference's cell maximum

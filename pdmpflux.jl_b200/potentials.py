@@ -93,8 +93,14 @@ class CudaPotential(Potential):
     when each sampler is built (CompileError carries the compiler log) and the sampler's kernels right after it.
     Compiled kernels are cached per process by source, so samplers that only change `params` do not compile again.
 
-    `accum` must be linear in x_i; the library cannot check it.  Every sampler runs a CudaPotential on its generic
-    kernel; RV_diagnostic does not (the contract has no U value)."""
+    Optional members declare the line model of the built-in plugins: `static constexpr bool affine` (constant Hessian
+    beyond the first `special` coordinates), `static constexpr int special` (coordinates that are their own
+    functionals) and the split line sums `eval_local` / `line_corr`.  A declared potential runs on the fast-path kernels
+    of Zig-Zag, BPS and ForwardECMC (Boomerang keeps the generic kernel); without them every sampler runs the generic
+    kernel.  RV_diagnostic does not run a CudaPotential (the contract has no U value).
+
+    `accum` must be linear in x_i, and a declared line model must hold exactly; the library can check neither, and a
+    wrong declaration samples the wrong target."""
     kind = SOURCE
 
     def __init__(self, source, params=()):
