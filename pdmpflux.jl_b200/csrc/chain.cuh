@@ -43,6 +43,18 @@ extern __shared__ __align__(128) double g_smem[];
 #define BOX(k) g_smem[off_box + (k) * kBStr]
 #define CUM(k) g_smem[off_cum + (k) * kBStr]
 
+// Phase clock of the thinning loop (tools/phase_clock.py).  Only a build with -DPDMPFLUX_PHASE_CLOCK has it: every
+// lane adds the clock64() cycles since its previous mark to the phase the mark closes, and run_events() adds its
+// lane's totals (and its event count) to g_phase_clock.  kPhIdle collects the cycles a lane spends waiting while
+// other lanes of its warp run a block it skips.  The default build compiles the marks to nothing.
+#ifdef PDMPFLUX_PHASE_CLOCK
+enum { kPhFunc, kPhPass, kPhReplay, kPhNext, kPhRate, kPhFlip, kPhIdle, kPhases };
+__device__ unsigned long long g_phase_clock[kPhases + 1];
+#define PDMPFLUX_PHASE(k) phase_mark(k)
+#else
+#define PDMPFLUX_PHASE(k) ((void)0)
+#endif
+
 // PATH selects how the bound and the rates are evaluated:
 //   kPathGeneric   every grid node / Brent iterate makes a pass over the coordinates (any potential, any option)
 //   kPathFastBrent affine line model + Brent (grid_size = 0)
@@ -146,6 +158,15 @@ struct Chain {
     bool exhausted;
 
     __device__ Chain(const KernelParams& p_) : p(p_) {}
+
+#ifdef PDMPFLUX_PHASE_CLOCK
+    long long ph_t, ph_acc[kPhases];
+    __device__ __forceinline__ void phase_mark(int k) {
+        const long long t = clock64();
+        ph_acc[k] += t - ph_t;
+        ph_t = t;
+    }
+#endif
 
     // ------------------------------------------------------------------------------------------------
     // draws: tape (parity mode) or Philox
@@ -1265,6 +1286,7 @@ struct Chain {
         s.x = __dadd_rn(s.lo, __dmul_rn(kGolden, __dadd_rn(s.hi, -s.lo)));
         s.fx = -rate_unsigned(s.x);
         s.stp = 0.0; s.old = 0.0; s.w = s.x; s.v = s.x; s.fw = s.fx; s.fv = s.fx;
+        PDMPFLUX_PHASE(kPhFunc);
         if constexpr (kTeamSpec) {
             // Transposed passes: lane tl of the team takes iterations tl, tl + TEAM, tl + 2 TEAM, ... of the next
             // kSuper * TEAM iterations -- on BASELINE config C2 a whole bound (36 iterations) is one pass.  While golden
@@ -1278,6 +1300,12 @@ struct Chain {
             // whose stopping rule fires ends the search, provided every iteration before it is vouched for by its lane.
             // Otherwise TEAM iterations are replayed one at a time and the next pass starts from there.  The operations
             // and operands of every iteration are the one-at-a-time recurrence's, so the result is bit-identical.
+            // A "tol step" -- golden step too short, |gstp| < tol, so u = x +- tol; on C2 the last step of nearly every
+            // bound -- moves (lo, hi, x) differently from what the recurrence predicts for the iterations after it, but
+            // its own lane knows the state it leaves: x = u, the bracket end on u's side unchanged, the other end x.
+            // So that lane also evaluates the stopping rule of the iteration after it.  When that fires (and the tol
+            // step is a new best in the assumed direction) the lane vouches for its iteration and sets the stop bit of
+            // the next one: the search ends on the tol step's value without replaying it.
             constexpr int S = kSuper;
             auto rot = [&](double v, int j) { return __shfl_sync(mask, v, (tl - j) & (TEAM - 1), TEAM); };
             bool done = false;
@@ -1308,7 +1336,7 @@ struct Chain {
                 }
                 double F[S], TOL[S], U[S];
                 unsigned long long stopmask = 0ull, goodmask = 0ull;
-                bool asok[S];
+                bool asok[S], tolok[S];
 #pragma unroll
                 for (int b = 0; b < S; ++b) {
                     const bool first = (b == 0) && (tl == 0);
@@ -1317,7 +1345,16 @@ struct Chain {
                     double mid, og, gstp;
                     U[b] = brent_golden(lo_, hi_, X[b], TOL[b], mid, og, gstp);
                     const bool stop = fabs(X[b] - mid) <= fma(hi_ - lo_, -0.5, TOL[b] + TOL[b]);
-                    asok[b] = ((X[b] < mid) == right) & (fabs(gstp) >= TOL[b]);
+                    const bool dir = (X[b] < mid) == right;
+                    asok[b] = dir & (fabs(gstp) >= TOL[b]);
+                    // tol step: the stopping rule of the next iteration, from the state this one leaves when it is a
+                    // new best (not at the pass's last iteration, whose successor belongs to the next pass)
+                    const double lo2 = right ? X[b] : lo_, hi2 = right ? hi_ : X[b];
+                    double tol2, mid2, og2, gstp2;
+                    brent_golden(lo2, hi2, U[b], tol2, mid2, og2, gstp2);
+                    const bool stop2 = fabs(U[b] - mid2) <= fma(hi2 - lo2, -0.5, tol2 + tol2);
+                    tolok[b] = dir & (fabs(gstp) < TOL[b]) & ((U[b] < X[b]) != right) & stop2 &
+                               (b < S - 1 || tl < TEAM - 1);
                     stopmask |= (unsigned long long)(stop ? 1u : 0u) << (TEAM * b + tl);   // my bits; merged below
                 }
                 rate_unsigned_n<S>(U, F);   // the S rates side by side (bit-identical to S calls of rate_unsigned)
@@ -1348,8 +1385,10 @@ struct Chain {
                         m.old = first ? s.old : E - W[b];
                         double pp, qq;
                         const bool para = brent_parabola(m, TOL[b], pp, qq);
-                        const bool good = !para & (F[b] < m.fx) & asok[b];
-                        goodmask |= (unsigned long long)(good ? 1u : 0u) << (TEAM * b + tl);
+                        const bool best = !para & (F[b] < m.fx);
+                        const bool fin = best & tolok[b];   // a tol step after which the search stops
+                        goodmask |= (unsigned long long)(((best & asok[b]) | fin) ? 1u : 0u) << (TEAM * b + tl);
+                        stopmask |= (unsigned long long)(fin ? 1u : 0u) << (TEAM * b + tl + 1);
                     }
                 }
                 stopmask = team_or64<TEAM>(stopmask, mask);
@@ -1367,6 +1406,7 @@ struct Chain {
                     return team_bcast<TEAM>(sel, step & (TEAM - 1), mask);
                 };
                 it += nc;
+                PDMPFLUX_PHASE(kPhPass);
                 if (nterm <= nbad && nterm < N) {   // the stopping rule fired: only the best value is needed
                     if (nterm >= 1) s.fx = at(F, nterm - 1);
                     done = true;
@@ -1392,7 +1432,9 @@ struct Chain {
                         }
                     }
                 }
+                PDMPFLUX_PHASE(kPhReplay);
             }
+            PDMPFLUX_PHASE(kPhIdle);
         } else if constexpr (kSpecB > 0) {
             bool done = false;
             for (int it = 0; it < 1000 && !done;) {
@@ -2037,6 +2079,11 @@ struct Chain {
         };
         accept = false;
         begin_event(0);
+#ifdef PDMPFLUX_PHASE_CLOCK
+        ph_t = clock64();
+#pragma unroll
+        for (int k = 0; k < kPhases; ++k) ph_acc[k] = 0;
+#endif
         // time-horizon variant: `while state.t < T` (src/sample.jl:360)
         if (p.use_t_stop && status == 0 && !(t < p.t_stop)) status = PDMPFLUX_CHAIN_DONE;
         bool live = valid && status == 0 && p.n_events > 0;
@@ -2044,6 +2091,7 @@ struct Chain {
         // head is the reconvergence point of each iteration, and both blocks of the body are plain ifs, so the
         // lanes that build a bound do it together and the lanes that have a proposal test it together.
         while (__any_sync(0xffffffffu, live)) {
+            PDMPFLUX_PHASE(kPhIdle);
             if (live && need_build) {
                 if (++steps > p.max_steps) { status = PDMPFLUX_CHAIN_STEP_LIMIT; live = false; }
                 else {
@@ -2059,6 +2107,7 @@ struct Chain {
                     const double e = rand_exp();
                     next_event(e, tp, lambda_bar);
                     exp_rv = e;
+                    PDMPFLUX_PHASE(kPhNext);
                     if (exhausted) { status = PDMPFLUX_CHAIN_TAPE_EXHAUSTED; live = false; }
                     else if (half) {
                         // QUIRK: a non-adaptive chain keeps the full horizon although the live bound covers half of it
@@ -2080,6 +2129,7 @@ struct Chain {
                     } else need_build = false;
                 }
             }
+            PDMPFLUX_PHASE(kPhIdle);
             if (live && !need_build) {
                 // moves_until_horizon!, :103-111: `while tp < horizon && !accept` -- otherwise a fresh outer step
                 if (!(tp < horizon)) need_build = true;
@@ -2088,8 +2138,10 @@ struct Chain {
                     ++n_rates;
                     const double lt = rate_unsigned(tp);
                     ar = lt / lambda_bar;
+                    PDMPFLUX_PHASE(kPhRate);
                     if (ar > 1.0) { need_build = true; half = true; }
                     else if (rand_uniform() < ar) {  // ac_step_with_proxy!, :153-168 -> if_accept!, :170-186
+                        PDMPFLUX_PHASE(kPhRate);
                         if (p.use_t_stop && t + tp + ts > p.t_stop) {
                             // The event falls beyond T: the skeleton ends with the point at exactly t = T reached by
                             // the deterministic flow, with zeroed event statistics (src/sample.jl:385-420).  The
@@ -2131,7 +2183,9 @@ struct Chain {
                             if (p.use_t_stop && !(t < p.t_stop)) { status = PDMPFLUX_CHAIN_DONE; live = false; }
                         }
                         }
+                        PDMPFLUX_PHASE(kPhFlip);
                     } else {  // if_reject!, :188-203
+                        PDMPFLUX_PHASE(kPhRate);
                         const double e3 = exp_rv + rand_exp();
                         next_event(e3, tp, lambda_bar);
                         horizon = p.adaptive ? horizon / 1.04 : horizon;  // QUIRK: shrink before the horizon check
@@ -2144,6 +2198,7 @@ struct Chain {
                             hh += 1;
                             need_build = true;
                         }
+                        PDMPFLUX_PHASE(kPhNext);
                     }
                 }
             }
@@ -2151,6 +2206,13 @@ struct Chain {
         if constexpr (kDefer) {
             if (pend != 0.0) flow_inplace(pend);  // a chain stopped inside an event: its stored state is the moved point
         }
+#ifdef PDMPFLUX_PHASE_CLOCK
+        if (valid) {
+#pragma unroll
+            for (int k = 0; k < kPhases; ++k) atomicAdd(&g_phase_clock[k], (unsigned long long)ph_acc[k]);
+            atomicAdd(&g_phase_clock[kPhases], (unsigned long long)ev);
+        }
+#endif
         return ev;
     }
 
