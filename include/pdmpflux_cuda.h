@@ -27,7 +27,8 @@
 extern "C" {
 #endif
 
-#define PDMPFLUX_VERSION 200 /* 0.2.0: pdmpflux_history gained is_active (appended), Sticky Zig-Zag, reductions */
+#define PDMPFLUX_VERSION 200 /* 0.2.1: potential kind PDMPFLUX_GAUSS_DENSE (appended; no layout change); 0.2.0:
+                                 pdmpflux_history gained is_active (appended), Sticky Zig-Zag, reductions */
 
 typedef enum pdmpflux_error {
     PDMPFLUX_OK = 0,
@@ -57,12 +58,19 @@ typedef enum pdmpflux_sampler_kind {
  *   BANANA_README_SCALAR -                      README.md:62-65 (scalar "gradient" broadcast to all coords)
  *   LOGREG               n, sigma0, X[n*d] row-major, y[n]
  *   SOURCE               p[n_params]            user-written CUDA source (pdmpflux_potential_create_source)
- * (A dense-precision Gaussian is not offered: the only "slanted" Gaussian BASELINE names is GAUSS_EQUICORR.)
+ *   GAUSS_DENSE          P[d*d] row-major, mu[d] U = (x - mu)' P (x - mu) / 2, P symmetric positive definite
+ * GAUSS_DENSE: P must be finite, symmetric to 1e-12 max|P| (it is stored as (P + P')/2) and positive definite
+ * (ERR_ARGUMENT otherwise); d <= 2048 (ERR_UNSUPPORTED above).  It runs on Zig-Zag and BPS only, on the configurations
+ * with a fast-path kernel: Zig-Zag needs a Brent bound (grid_size = 0) or a vectorised grid bound with an exact
+ * AD_backend; every BPS configuration qualifies.  Anything else is ERR_UNSUPPORTED at sampler creation.  The chains
+ * keep g = P (x - mu) and h = P v next to x and v and update them per event (a Zig-Zag flip reads one row of P, a BPS
+ * reflection or refresh all of it).  pdmpflux_rv_diagnostic does not run it (ERR_UNSUPPORTED).
  */
 typedef enum pdmpflux_potential_kind {
     PDMPFLUX_GAUSS_STD = 0, PDMPFLUX_GAUSS_DIAG = 1, PDMPFLUX_GAUSS_EQUICORR = 2, PDMPFLUX_BANANA = 3,
     PDMPFLUX_BANANA_README_SCALAR = 4, PDMPFLUX_LOGREG = 5,
-    PDMPFLUX_SOURCE = 6 /* created by pdmpflux_potential_create_source only */
+    PDMPFLUX_SOURCE = 6, /* created by pdmpflux_potential_create_source only */
+    PDMPFLUX_GAUSS_DENSE = 7
 } pdmpflux_potential_kind;
 
 /* How d/dt of the rate is obtained on the time grid: JVP = analytic (what AD_backend="ForwardDiff" computes,

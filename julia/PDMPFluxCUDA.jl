@@ -10,7 +10,7 @@ module PDMPFluxCUDA
 import PDMPFlux
 import PDMPFlux: PDMPHistory, sample_skeleton, sample_from_skeleton, sample, RV_diagnostic,
                  sample_skeleton_with_diagnostic
-export CuPotential, GaussStd, GaussDiag, GaussEquicorr, Banana, BananaReadmeScalar, LogReg, CudaPotential, CuPDMP, CuHistoryBatch,
+export CuPotential, GaussStd, GaussDiag, GaussEquicorr, GaussDense, Banana, BananaReadmeScalar, LogReg, CudaPotential, CuPDMP, CuHistoryBatch,
        moments_reduce, CuComm, comm_unique_id, moments_allreduce!
 
 const LIB = get(ENV, "PDMPFLUX_CUDA_LIB", joinpath(@__DIR__, "..", "pdmpflux.jl_b200", "lib", "libpdmpflux_cuda.so"))
@@ -52,6 +52,9 @@ CuPotential(kind::Integer, params::Vector{Float64}) = CuPotential(Int32(kind), p
 GaussStd() = CuPotential(0, Float64[])
 GaussDiag(p::AbstractVector) = CuPotential(1, collect(Float64, p))
 GaussEquicorr(rho::Real) = CuPotential(2, [Float64(rho)])
+# U = (x - mu)' P (x - mu) / 2, P dense symmetric positive definite (checked by the library); Zig-Zag and BPS only
+GaussDense(P::AbstractMatrix, mu::AbstractVector = zeros(size(P, 1))) =
+    CuPotential(7, vcat(vec(permutedims(Float64.(P))), Float64.(mu)))
 Banana() = CuPotential(3, Float64[])
 BananaReadmeScalar() = CuPotential(4, Float64[])
 "Bayesian logistic regression posterior: rows of `X` (n × d), labels `y` in {0, 1}, prior N(0, sigma0² I).  X is

@@ -10,7 +10,8 @@ from ._lib import (ArgumentError, CapacityError, ChainError, CompileError, CudaE
 from .device import DeviceChains, device_history_view
 from . import dist
 from .history import PDMPHistory, PDMPHistoryBatch
-from .potentials import (Banana, BananaReadmeScalar, CudaPotential, GaussDiag, GaussEquicorr, GaussStd, LogReg, Potential)
+from .potentials import (Banana, BananaReadmeScalar, CudaPotential, GaussDense, GaussDiag, GaussEquicorr, GaussStd, LogReg,
+                         Potential)
 from .sample import (RV_diagnostic, ess_from_chain_means, sample, sample_from_skeleton, sample_skeleton,
                      sample_skeleton_until, sample_skeleton_with_diagnostic, skeleton_moments)
 from .samplers import (BPS, BPSAD, AbstractPDMP, Boomerang, BoomerangAD, ForwardECMC, ForwardECMCAD, SpeedUpZigZag,
@@ -21,7 +22,7 @@ __all__ = [
     "StickyZigZagAD", "SpeedUpZigZag", "SpeedUpZigZagAD",
     "AbstractPDMP", "sample", "sample_skeleton", "RV_diagnostic", "sample_skeleton_with_diagnostic", "sample_skeleton_until", "CapacityError", "sample_from_skeleton", "skeleton_moments",
     "ess_from_chain_means", "PDMPHistory", "PDMPHistoryBatch", "Potential", "GaussStd", "GaussDiag",
-    "GaussEquicorr", "Banana", "BananaReadmeScalar", "LogReg", "CudaPotential", "ArgumentError", "DimensionMismatch",
+    "GaussEquicorr", "GaussDense", "Banana", "BananaReadmeScalar", "LogReg", "CudaPotential", "ArgumentError", "DimensionMismatch",
     "UnsupportedError", "CudaError", "ChainError", "CompileError", "build", "lib", "LIB_PATH", "DeviceChains",
     "device_history_view", "dist",
 ]

@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
@@ -72,6 +73,10 @@ struct pdmpflux_potential_s {
     DevBuf params;
     std::string source;  // PDMPFLUX_SOURCE: the user's CUDA text (jit.cu)
     SourceTraits traits; // PDMPFLUX_SOURCE: the line model it declares (read by the contract check)
+    // GAUSS_DENSE: the validated (P + P')/2 and mu, uploaded into `params` when the first chains are created (so that a
+    // potential and its samplers can be built and checked without a device)
+    std::vector<double> host;
+    std::mutex upload_mu;
 };
 
 // Device slabs of the host-buffer pipeline, cached in the sampler handle so that repeated sample_skeleton calls do
@@ -123,6 +128,7 @@ struct pdmpflux_chains_s {
     unsigned grid = 0;
     int64_t n_groups = 0;   // groups of chains (one block's worth); grid < n_groups: persistent blocks walk over the groups
     DevBuf x, v, t, horizon, ar, tape_pos, status, counters, scratch, ncols, m1, m2, wq, act;
+    DevBuf g, h;  // dense Gaussian: g = P (x - mu), h = P v
     int moments = 0;
     double t_stop = 0.0;
     int use_t_stop = 0;
@@ -168,11 +174,11 @@ int default_team(int d, int64_t n_chains, bool zz_brent_fast) {
 
 // widen the team until the per-thread-owned shared-memory columns of a block (x, v, Zig-Zag x Brent A / B, moments,
 // sticky flags; ForwardECMC scratch goes to global memory when it is large) leave room for a second block
-int widen_team(int team, int sampler, int path, int d) {
+int widen_team(int team, int sampler, int path, int d, int pot) {
     auto vectors_bytes = [&](int team) {
-        const int bt_ = block_threads_rt(team, sampler, path);
+        const int bt_ = block_threads_rt(team, sampler, path, pot);
         const int n_own = (d + team - 1) / team;
-        const size_t nv = state_vectors(sampler, path, team, brent_line_model(sampler, path, team, n_own));
+        const size_t nv = state_vectors(sampler, path, team, brent_line_model(sampler, path, team, n_own, pot), pot);
         return (nv + 2 /* fused moments may be enabled later */ + (sampler == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) *
                (size_t)n_own * bt_ * sizeof(double);
     };
@@ -196,13 +202,16 @@ struct Variant { int path, team, n_own, nw; };
 Variant chain_variant(int kind, int dim, const pdmpflux_config& cfg, const pdmpflux_potential_s* pot, int64_t n_chains,
                       bool with_env) {
     Variant v{};
+    // the dense Gaussian has fast-path kernels on teams only: no generic kernel, no thread per chain
+    const bool dense = pot->kind == PDMPFLUX_GAUSS_DENSE;
     v.path = select_path(kind, line_traits(kind, pot), cfg.grid_size, cfg.vectorized_bound, cfg.deriv_mode);
-    if (const char* e = with_env ? std::getenv("PDMPFLUX_FORCE_GENERIC") : nullptr) { if (std::atoi(e)) v.path = kPathGeneric; }
+    if (const char* e = with_env && !dense ? std::getenv("PDMPFLUX_FORCE_GENERIC") : nullptr) { if (std::atoi(e)) v.path = kPathGeneric; }
     const bool zz_brent_fast = kind == PDMPFLUX_ZIGZAG && v.path == kPathFastBrent && pot->kind != PDMPFLUX_LOGREG;
-    const int team = with_env ? pick_team(dim, n_chains, zz_brent_fast) : default_team(dim, n_chains, zz_brent_fast);
-    v.team = widen_team(team, kind, v.path, dim);
+    int team = with_env ? pick_team(dim, n_chains, zz_brent_fast) : default_team(dim, n_chains, zz_brent_fast);
+    if (dense && team == 1) team = 8;
+    v.team = widen_team(team, kind, v.path, dim, pot->kind);
     v.n_own = (dim + v.team - 1) / v.team;
-    v.nw = brent_line_model(kind, v.path, v.team, v.n_own);
+    v.nw = brent_line_model(kind, v.path, v.team, v.n_own, pot->kind);
     return v;
 }
 
@@ -247,6 +256,7 @@ int launch(pdmpflux_chains_s* ch, int64_t n_events, const pdmpflux_history* h, i
     p.kappa = s->kappa.as<double>(); p.sact = ch->act.as<uint8_t>(); p.ACT = h ? h->is_active : nullptr;
     p.scratch = ch->scratch.as<double>(); p.scratch_in_smem = ch->scratch_in_smem; p.n_own = ch->n_own;
     p.brent_nw = ch->brent_nw;
+    p.sg = ch->g.as<double>(); p.sh = ch->h.as<double>();
     p.vec_elems = ch->vec_elems; p.dpad = ch->dpad;
     if (h) {
         auto al = [](const void* q, uintptr_t a) { return q == nullptr || (reinterpret_cast<uintptr_t>(q) % a) == 0; };
@@ -461,6 +471,80 @@ __global__ void __launch_bounds__(256, FLOW == 1 ? 4 : 6) moments_kernel(int d, 
     if (a == 0 && Tlen) Tlen[c] = t[n_sk - 1] - t[col_begin];
 }
 
+// GAUSS_DENSE parameters: P (d x d, row-major) then mu (d).  P must be finite, symmetric to 1e-12 max|P| and positive
+// definite (host Cholesky); out = (P + P')/2 followed by mu.  d <= kDenseMaxDim keeps P (32 MB) resident in the L2.
+constexpr int kDenseMaxDim = 2048;
+int dense_validate(int d, const double* params, int64_t n_params, std::vector<double>& out) {
+    if (d > kDenseMaxDim)
+        return fail(PDMPFLUX_ERR_UNSUPPORTED, "GAUSS_DENSE supports dim <= " + std::to_string(kDenseMaxDim) + " (P must stay L2-resident)");
+    const size_t dd = (size_t)d * d;
+    if (!params || n_params < (int64_t)(dd + d)) return fail(PDMPFLUX_ERR_ARGUMENT, "GAUSS_DENSE needs P[d*d] (row-major) and mu[d]");
+    double amax = 0.0;
+    for (size_t k = 0; k < dd + d; ++k) {
+        if (!std::isfinite(params[k])) return fail(PDMPFLUX_ERR_ARGUMENT, "GAUSS_DENSE: P and mu must be finite");
+        if (k < dd) amax = std::max(amax, std::fabs(params[k]));
+    }
+    out.assign(params, params + dd + d);
+    for (int i = 0; i < d; ++i)
+        for (int j = i + 1; j < d; ++j) {
+            const double a = params[(size_t)i * d + j], b = params[(size_t)j * d + i];
+            if (std::fabs(a - b) > 1e-12 * amax) return fail(PDMPFLUX_ERR_ARGUMENT, "GAUSS_DENSE: the precision matrix P is not symmetric");
+            out[(size_t)i * d + j] = out[(size_t)j * d + i] = 0.5 * (a + b);
+        }
+    // Cholesky P = L L' (L row-major, lower): every inner product runs over two contiguous rows
+    std::vector<double> L(dd, 0.0);
+    for (int j = 0; j < d; ++j) {
+        const double* lj = L.data() + (size_t)j * d;
+        double s = out[(size_t)j * d + j];
+        for (int k = 0; k < j; ++k) s -= lj[k] * lj[k];
+        if (!(s > 0.0)) return fail(PDMPFLUX_ERR_ARGUMENT, "GAUSS_DENSE: the precision matrix P is not positive definite");
+        const double ljj = std::sqrt(s);
+        L[(size_t)j * d + j] = ljj;
+        for (int i = j + 1; i < d; ++i) {
+            const double* li = L.data() + (size_t)i * d;
+            double t = out[(size_t)i * d + j];
+            for (int k = 0; k < j; ++k) t -= li[k] * lj[k];
+            L[(size_t)i * d + j] = t / ljj;
+        }
+    }
+    return PDMPFLUX_OK;
+}
+
+// GAUSS_DENSE: upload P and mu on first use (once per potential; samplers on several threads may share it)
+int dense_upload(pdmpflux_potential_s* pot) {
+    std::lock_guard<std::mutex> lock(pot->upload_mu);
+    if (pot->params.p) return PDMPFLUX_OK;
+    const size_t bytes = sizeof(double) * pot->host.size();
+    if (pot->params.alloc(bytes) != cudaSuccess || cudaMemcpy(pot->params.p, pot->host.data(), bytes, cudaMemcpyHostToDevice) != cudaSuccess) {
+        pot->params.alloc(0);
+        return fail(PDMPFLUX_ERR_CUDA, "GAUSS_DENSE parameter upload failed");
+    }
+    pot->pp.vec = pot->params.as<double>();
+    pot->pp.vec2 = pot->pp.vec + (size_t)pot->dim * pot->dim;
+    return PDMPFLUX_OK;
+}
+
+// dense Gaussian: g = P (x - mu) and h = P v of every chain (chains_create).  Chains on grid.x, one thread per
+// coordinate i: the threads of a block read consecutive entries of row k of P (= column k, P symmetric), x_k and v_k
+// are broadcasts.
+__global__ void __launch_bounds__(256) dense_state_kernel(int d, const double* __restrict__ P, const double* __restrict__ mu,
+                                                          const double* __restrict__ x, const double* __restrict__ v,
+                                                          double* __restrict__ g, double* __restrict__ h) {
+    const int64_t c = blockIdx.x;
+    const int i = blockIdx.y * blockDim.x + threadIdx.x;
+    if (i >= d) return;
+    const double* xc = x + c * d;
+    const double* vc = v + c * d;
+    double sg = 0.0, sh = 0.0;
+    for (int k = 0; k < d; ++k) {
+        const double pki = P[(size_t)k * d + i];
+        sg = fma(pki, xc[k] - mu[k], sg);
+        sh = fma(pki, vc[k], sh);
+    }
+    g[c * d + i] = sg;
+    h[c * d + i] = sh;
+}
+
 int normalise_config(int kind, int dim, pdmpflux_config& c) {
     // constructor rewrites: ZigZagSamplers.jl:73-78, BouncyParticleSamplers.jl:29-37,
     // ForwardEventChainMonteCarlo.jl:306-323, BoomerangSamplers.jl:27-36
@@ -552,6 +636,7 @@ int pdmpflux_potential_create(int kind, int dim, const double* params, int64_t n
     case PDMPFLUX_SOURCE:
         rc = fail(PDMPFLUX_ERR_ARGUMENT, "PDMPFLUX_SOURCE potentials carry CUDA source: create them with pdmpflux_potential_create_source");
         break;
+    case PDMPFLUX_GAUSS_DENSE: rc = dense_validate(dim, params, n_params, pot->host); break;
     default: rc = fail(PDMPFLUX_ERR_ARGUMENT, "unknown potential kind " + std::to_string(kind));
     }
     if (rc != PDMPFLUX_OK) { delete pot; return rc; }
@@ -615,6 +700,18 @@ static int sampler_create_impl(int kind, int dim, pdmpflux_potential_t pot, cons
     if (!(cfg->tmax >= 0.0) || !std::isfinite(cfg->tmax)) return fail(PDMPFLUX_ERR_ARGUMENT, "tmax must be finite and >= 0");
     pdmpflux_config ncfg = *cfg;
     normalise_config(kind, dim, ncfg);
+    if (pot->kind == PDMPFLUX_GAUSS_DENSE) {  // fast-path kernels only: no generic kernel, no CPU fallback
+        const char* what = nullptr;
+        if (kind != PDMPFLUX_ZIGZAG && kind != PDMPFLUX_BPS)
+            what = kind == PDMPFLUX_FECMC ? "ForwardECMC" : kind == PDMPFLUX_BOOMERANG ? "Boomerang"
+                 : kind == PDMPFLUX_STICKY_ZIGZAG ? "StickyZigZag" : "SpeedUpZigZag";
+        else if (select_path(kind, builtin_line_traits(pot->kind), ncfg.grid_size, ncfg.vectorized_bound, ncfg.deriv_mode) == kPathGeneric)
+            what = !ncfg.vectorized_bound ? "ZigZag with vectorized_bound=false and a grid bound"
+                                          : "ZigZag with a grid bound and AD_backend=FiniteDiff";
+        if (what)
+            return fail(PDMPFLUX_ERR_UNSUPPORTED, std::string("GAUSS_DENSE runs on the ZigZag and BPS fast-path kernels only: ") + what +
+                                                      " is not supported (use grid_size=0, or a vectorised grid bound with an exact AD_backend)");
+    }
     if (pot->kind == PDMPFLUX_SOURCE) {
         // compile every kernel variant the default policy can pick for this sampler (the team widths chosen at one
         // chain and at any number of chains) before any CUDA call, so that source errors surface here even without a
@@ -683,7 +780,7 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
         const int rc = jit_prepare(s->pot->source, s->kind, ch->team, ch->path, ch->brent_nw);
         if (rc != PDMPFLUX_OK) return rc;
     }
-    const int bt = block_threads_rt(ch->team, s->kind, ch->path);   // threads per block of the kernel that will run
+    const int bt = block_threads_rt(ch->team, s->kind, ch->path, s->pot->kind);   // threads per block of the kernel that will run
     const int cpb = bt / ch->team;
     ch->grid = (unsigned)((n_chains + cpb - 1) / cpb);
     ch->n_groups = ch->grid;
@@ -694,7 +791,7 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
         ch->vec_elems = cpb * ch->dpad;
     }
     const size_t vec_bytes = (size_t)ch->vec_elems * sizeof(double);
-    const size_t nvec = state_vectors(s->kind, ch->path, ch->team, ch->brent_nw);
+    const size_t nvec = state_vectors(s->kind, ch->path, ch->team, ch->brent_nw, s->pot->kind);
     ch->smem = (nvec + (s->kind == PDMPFLUX_STICKY_ZIGZAG ? 1 : 0)) * vec_bytes;
     const size_t list_slack = ch->brent_nw == kLineTransposed ? 16 * sizeof(double) : 0;   // transposed Brent: unconditional reads of the 12-slot list
     if (s->kind == PDMPFLUX_FECMC) {
@@ -752,6 +849,16 @@ int pdmpflux_chains_create(pdmpflux_sampler_t s, int64_t n_chains, const double*
     const cudaMemcpyKind k = init_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     CUDA_TRY(cudaMemcpy(ch->x.p, xinit, sizeof(double) * d * n_chains, k));
     CUDA_TRY(cudaMemcpy(ch->v.p, vinit, sizeof(double) * d * n_chains, k));
+    if (s->pot->kind == PDMPFLUX_GAUSS_DENSE) {
+        const int rc = dense_upload(s->pot);
+        if (rc != PDMPFLUX_OK) return rc;
+        CUDA_TRY(ch->g.alloc(sizeof(double) * d * n_chains));
+        CUDA_TRY(ch->h.alloc(sizeof(double) * d * n_chains));
+        dense_state_kernel<<<dim3((unsigned)n_chains, (unsigned)((d + 255) / 256)), 256>>>(
+            d, s->pot->pp.vec, s->pot->pp.vec2, ch->x.as<double>(), ch->v.as<double>(), ch->g.as<double>(), ch->h.as<double>());
+        CUDA_TRY(cudaGetLastError());
+        g_launches.fetch_add(1);
+    }
     CUDA_TRY(cudaMemset(ch->t.p, 0, sizeof(double) * n_chains));
     CUDA_TRY(cudaMemset(ch->ar.p, 0, sizeof(double) * n_chains));
     CUDA_TRY(cudaMemset(ch->tape_pos.p, 0, sizeof(int64_t) * 3 * n_chains));
@@ -1399,6 +1506,8 @@ int pdmpflux_rv_diagnostic(pdmpflux_potential_t pot, int flow_kind, int64_t n_sk
         return fail(PDMPFLUX_ERR_ARGUMENT, "invalid argument");
     if (pot->kind == PDMPFLUX_SOURCE)
         return fail(PDMPFLUX_ERR_UNSUPPORTED, "RV_diagnostic needs U(x), which a source potential does not define (it gives grad U only)");
+    if (pot->kind == PDMPFLUX_GAUSS_DENSE)
+        return fail(PDMPFLUX_ERR_UNSUPPORTED, "RV_diagnostic has no value kernel for GAUSS_DENSE");
     if (B < 0) return fail(PDMPFLUX_ERR_ARGUMENT, "B must be non-negative");  // diagnostic.jl:49-51
     if (flow_kind != 0 && flow_kind != 1) return fail(PDMPFLUX_ERR_ARGUMENT, "flow_kind must be 0 (linear) or 1 (rotation)");
     int ndev = 0;

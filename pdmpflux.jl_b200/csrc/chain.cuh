@@ -34,6 +34,9 @@ extern __shared__ __align__(128) double g_smem[];
 #define VS(j) g_smem[off_v + (j) * kStr]
 #define AS(j) g_smem[off_a + (j) * kStr]
 #define BS(j) g_smem[off_b + (j) * kStr]
+// dense Gaussian: the maintained g = P (x - mu) and h = P v of the owned coordinates
+#define GS(j) g_smem[off_g + (j) * kStr]
+#define HS(j) g_smem[off_h + (j) * kStr]
 #define M1S(j) g_smem[off_m1 + (j) * kStr]
 #define M2S(j) g_smem[off_m2 + (j) * kStr]
 // Sticky Zig-Zag: 1.0 / 0.0 activity flag per coordinate; VU = the velocity the flow, the rates and the bounds see
@@ -96,7 +99,15 @@ struct Chain {
     static constexpr bool kZZ = (SAMPLER == PDMPFLUX_ZIGZAG) || kSticky || kSpeedUp;   // StickyZigZagSamplers.jl:69-101: same closures
     static_assert(!kSticky || PATH == kPathGeneric, "Sticky Zig-Zag runs on the generic path");
     static_assert(!kSpeedUp || PATH == kPathGeneric, "Speed-Up Zig-Zag runs on the generic path");
-    static constexpr int kBT = block_threads_rt(TEAM, SAMPLER, PATH);   // threads per block
+    // Dense Gaussian (Pot<PDMPFLUX_GAUSS_DENSE>): the chain keeps g = P (x - mu) and h = P v in shared memory and
+    // updates them with every change of x or v -- a move by tau adds tau h to g, a Zig-Zag flip of coordinate m adds
+    // 2 v_m' P[m, :] to h (one row of P), a BPS reflection or refresh recomputes the change of h with one pass over P.
+    // Only the fast paths of Zig-Zag and BPS on teams with the shared-memory line model are built for it.
+    static constexpr bool kDense = (POT == PDMPFLUX_GAUSS_DENSE);
+    static_assert(!kDense || (PATH != kPathGeneric && TEAM > 1 && NW == kLineShared &&
+                              (SAMPLER == PDMPFLUX_ZIGZAG || SAMPLER == PDMPFLUX_BPS)),
+                  "the dense Gaussian runs on the Zig-Zag / BPS fast paths of teams with the shared line model");
+    static constexpr int kBT = block_threads_rt(TEAM, SAMPLER, PATH, POT);   // threads per block
     static constexpr int kStr = (TEAM == 1) ? kBT : TEAM;  // stride between a thread's owned elements
     static constexpr int kBStr = (TEAM == 1) ? kBT : 1;    // stride between a chain's box / cum entries
 
@@ -105,6 +116,7 @@ struct Chain {
     double tt;                       // Sticky Zig-Zag: time to thaw (StickySamplingLoop.jl:43)
     int off_m1, off_m2;              // fused-moment accumulators (owned columns, only when p.accumulate_moments)
     int off_x, off_v, off_a, off_b;  // element offsets into g_smem of this thread's owned columns of x, v, A, B
+    int off_g, off_h;                // dense Gaussian: ... of g = P (x - mu) and h = P v
     double* sc0; // scratch owned vectors (FECMC)
     double* sc1;
     double* sc2;
@@ -265,6 +277,23 @@ struct Chain {
         if (tl < d - TEAM * nfull) f(nfull);
     }
 
+    // Dense Gaussian: (P w)_i for the coordinate i of owned slot j, w = the chain's vector whose owned column starts at
+    // element offset off_w (its other coordinates are read from the chain-contiguous row, so the team must have synced
+    // after writing it).  P is symmetric: column i is read as row i's transpose, P[k, i] over k, so the lanes of a team
+    // read consecutive addresses of row k; w_k is a shared-memory broadcast.  P stays L2-resident (at most 32 MB).
+    __device__ __forceinline__ double dense_matvec(int j, int off_w) const {
+        const double* col = p.pot.vec + coord(j);
+        const double* w = g_smem + (off_w - tl);
+        double s[4] = {0.0, 0.0, 0.0, 0.0};
+        int k = 0;
+        for (; k + 3 < d; k += 4) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) s[u] = fma(__ldg(col + (size_t)(k + u) * d), w[k + u], s[u]);
+        }
+        for (; k < d; ++k) s[0] = fma(__ldg(col + (size_t)k * d), w[k], s[0]);
+        return (s[0] + s[1]) + (s[2] + s[3]);
+    }
+
     // functionals of the current x and v (one fused multi-value reduction)
     __device__ void compute_functionals() {
         if constexpr (K > 0) {
@@ -371,6 +400,7 @@ struct Chain {
             flow_point(f, XS(j), VU(j), xt, vt);
             XS(j) = xt;
             if constexpr (kRot) VS(j) = vt;
+            if constexpr (kDense) GS(j) = GS(j) + tt * HS(j);   // g(x + tt v) = g + tt P v
         });
     }
 
@@ -432,7 +462,8 @@ struct Chain {
                     if (owns(j) && coord(j) >= NS) {
                         const double vi = VS(j);
                         double g, hv;
-                        P::eval(p.pot, coord(j), XS(j), vi, Lx, Lv, g, hv);
+                        if constexpr (kDense) { g = GS(j); hv = HS(j); }
+                        else P::eval(p.pot, coord(j), XS(j), vi, Lx, Lv, g, hv);
                         A = g * vi; B = hv * vi;
                     }
                     AS(j) = A; BS(j) = B;
@@ -446,7 +477,8 @@ struct Chain {
                 for_owned([&](int j) {
                     const double vi = VS(j);
                     double gl, hl;
-                    P::eval_local(p.pot, coord(j), XS(j), vi, gl, hl);
+                    if constexpr (kDense) { gl = GS(j); hl = HS(j); }
+                    else P::eval_local(p.pot, coord(j), XS(j), vi, gl, hl);
                     r2[0] += gl * vi; r2[1] += hl * vi;
                 });
                 team_sum_n<TEAM, 2>(r2, mask);
@@ -597,7 +629,9 @@ struct Chain {
                 if (owns(j)) {
                     double xt, vt;
                     flow_point(f, XS(j), VU(j), xt, vt);
-                    const double y = grad_eff(P::grad(p.pot, coord(j), xt, Lxt), xt, f.sp) * vt;
+                    double y;
+                    if constexpr (kDense) y = (GS(j) + f.b * HS(j)) * vt;   // g(x + t v) = g + t h
+                    else y = grad_eff(P::grad(p.pot, coord(j), xt, Lxt), xt, f.sp) * vt;
                     if constexpr (kZZ) s += (y > 0.0 ? y : 0.0);
                     else s += y;
                 }
@@ -791,7 +825,8 @@ struct Chain {
                 // per (coordinate, cell), no compares or selects.
                 const double vi = VS(j);
                 double g, hv;
-                P::eval(p.pot, i, XS(j), vi, Lx, Lv, g, hv);
+                if constexpr (kDense) { g = GS(j); hv = HS(j); }
+                else P::eval(p.pot, i, XS(j), vi, Lx, Lv, g, hv);
                 const double A = g * vi, B = hv * vi, aB = fabs(B);
 #pragma unroll
                 for (int u = 0; u < kCellsV; ++u)
@@ -1611,6 +1646,7 @@ struct Chain {
             const double xn = XS(j) + VS(j) * T;
             XS(j) = xn;
             if constexpr (K > 0) P::accum(p.pot, coord(j), xn, ax);
+            if constexpr (kDense) GS(j) = GS(j) + T * HS(j);
         });
         if constexpr (K > 0) {
             team_sum_n<TEAM, KK>(ax, mask);
@@ -1619,7 +1655,9 @@ struct Chain {
         }
         double r2[2] = {0.0, 0.0};
         for_owned([&](int j) {
-            const double g = P::grad(p.pot, coord(j), XS(j), Lx);
+            double g;
+            if constexpr (kDense) g = GS(j);
+            else g = P::grad(p.pot, coord(j), XS(j), Lx);
             r2[0] += g * VS(j);
             r2[1] += g * g;
         });
@@ -1631,7 +1669,25 @@ struct Chain {
         if (u < prob) {
             if (gg == 0) return true;   // v unchanged: Lv still valid
             const double scale = 2 * gv / gg;
-            if constexpr (P::kSplit) {   // functionals AND line model of the new velocity in the pass that writes it
+            if constexpr (kDense) {
+                // v' = v - scale g, h' = P v' = h - scale (P g): one pass over P, fused with the write of v' and the line
+                // model of the new state (a = <g, v'>, b = <h', v'>)
+                __syncwarp(mask);  // g of the flow pass above is read chain-contiguously by dense_matvec
+                double av[2] = {0.0, 0.0};
+                for_owned<1>([&](int j) {
+                    const double g = GS(j);
+                    const double vn = VS(j) - scale * g;
+                    const double hn = HS(j) - scale * dense_matvec(j, off_g);
+                    VS(j) = vn; HS(j) = hn;
+                    av[0] += g * vn; av[1] += hn * vn;
+                });
+                team_sum_n<TEAM, 2>(av, mask);
+                double ca_, cb_;
+                P::line_corr(p.pot, Lx, Lv, ca_, cb_);   // the sums prepare_line() forms, bit for bit
+                la = av[0] + ca_; lb = av[1] + cb_;
+                line_ready = true;
+                return true;
+            } else if constexpr (P::kSplit) {   // functionals AND line model of the new velocity in the pass that writes it
                 double av[KK + 2];
 #pragma unroll
                 for (int k = 0; k < KK + 2; ++k) av[k] = 0.0;
@@ -1674,6 +1730,10 @@ struct Chain {
         if (!p.gaussian_velocity) {
             nn = 1.0 / sqrt(team_sum<TEAM>(nn, mask));
             for_owned([&](int j) { VS(j) = VS(j) * nn; });
+        }
+        if constexpr (kDense) {  // h = P v of the new velocity: one pass over P
+            __syncwarp(mask);
+            for_owned<1>([&](int j) { HS(j) = dense_matvec(j, off_v); });
         }
         return false;
     }
@@ -1997,13 +2057,19 @@ struct Chain {
             // lane, ONE scan over the lanes' block totals, and a short search inside the block that holds the index.
             __syncwarp(mask);  // x / v written under the strided ownership are visible to the whole team
             const int cbx = off_x - tl, cbv = off_v - tl;  // element offset of the chain's coordinate 0
+            const int cbg = off_g - tl, cbh = off_h - tl;  // (dense Gaussian: g, h)
             const int i0 = tl * nown, i1 = min(d, i0 + nown);
             double tot = 0.0;
             for (int i = i0; i < i1; ++i) {
                 const double vi = g_smem[cbv + i];
                 const double xn = g_smem[cbx + i] + vi * tt;
                 g_smem[cbx + i] = xn;
-                const double y = P::grad(p.pot, i, xn, Lxn) * vi;
+                double y;
+                if constexpr (kDense) {
+                    const double gn = g_smem[cbg + i] + tt * g_smem[cbh + i];
+                    g_smem[cbg + i] = gn;
+                    y = gn * vi;
+                } else y = P::grad(p.pot, i, xn, Lxn) * vi;
                 tot += (y > 0.0 ? y : 0.0);
             }
             const double incl = team_scan_incl<TEAM>(tot, mask, tl);
@@ -2011,19 +2077,29 @@ struct Chain {
             if (tl == 0) excl = 0.0;
             const unsigned b = team_ballot<TEAM>((i0 < i1) && (incl > uS), tl, mask);
             const int first = b ? (__ffs(b) - 1) : -1;
+            int m_dense = d - 1;
             if (first < 0) {  // rounding left the total below u S: the reference's scan ends on the last index
                 if (tl == (d - 1) / nown) g_smem[cbv + d - 1] = -g_smem[cbv + d - 1];
             } else if (tl == first) {
                 double cum = excl;
                 int m = i1 - 1;
                 for (int i = i0; i < i1; ++i) {
-                    const double y = P::grad(p.pot, i, g_smem[cbx + i], Lxn) * g_smem[cbv + i];
+                    double y;
+                    if constexpr (kDense) y = g_smem[cbg + i] * g_smem[cbv + i];
+                    else y = P::grad(p.pot, i, g_smem[cbx + i], Lxn) * g_smem[cbv + i];
                     cum += (y > 0.0 ? y : 0.0);
                     if (cum > uS) { m = i; break; }
                 }
                 g_smem[cbv + m] = -g_smem[cbv + m];
+                if constexpr (kDense) m_dense = m;
             }
             __syncwarp(mask);
+            if constexpr (kDense) {  // h = P v after v_m flipped: h += 2 v_m' P[m, :] (row m: coalesced over the lanes)
+                const int m = first < 0 ? d - 1 : __shfl_sync(mask, m_dense, first, TEAM);
+                const double two_vm = 2.0 * g_smem[cbv + m];
+                const double* row = p.pot.vec + (size_t)m * d;
+                for_owned([&](int j) { HS(j) = fma(two_vm, __ldg(row + coord(j)), HS(j)); });
+            }
         }
     }
 
@@ -2561,8 +2637,8 @@ struct Chain {
 // n_events == 0 and col0 names the column).  Grid = ceil(n_chains / (kBT / TEAM)).
 constexpr int kMinBlocksGrid = 4;   // grid-bound kernels of teams of 1 / 8: blocks per SM (3 measured -10 .. -13 %)
 template <int TEAM, int SAMPLER, int POT, int PATH, int NW = kLineShared>
-__global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH == kPathGeneric ? 1 : (PATH == kPathFastBrent ? (TEAM == 1 && SAMPLER == PDMPFLUX_ZIGZAG ? 4 : 2) : (TEAM == 32 ? 3 : kMinBlocksGrid))) skeleton_kernel(const __grid_constant__ KernelParams p) {
-    constexpr int kBT = block_threads_rt(TEAM, SAMPLER, PATH);
+__global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH, POT), PATH == kPathGeneric ? 1 : (PATH == kPathFastBrent ? (TEAM == 1 && SAMPLER == PDMPFLUX_ZIGZAG ? 4 : 2) : (TEAM == 32 ? 3 : kMinBlocksGrid))) skeleton_kernel(const __grid_constant__ KernelParams p) {
+    constexpr int kBT = block_threads_rt(TEAM, SAMPLER, PATH, POT);
     constexpr int CPB = kBT / TEAM;  // chains per block
     const int c_local = threadIdx.x / TEAM;
     // A block normally owns one group of CPB chains (grid = number of groups).  With p.n_groups > gridDim.x the grid is
@@ -2589,12 +2665,17 @@ __global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH ==
     const int toff = (TEAM == 1) ? (int)threadIdx.x : c_local * p.dpad + ch.tl;  // this thread's offset in a vector
     ch.off_x = toff;
     ch.off_v = vec + toff;
-    constexpr int kVectors = state_vectors(SAMPLER, PATH, TEAM, NW);
+    constexpr int kVectors = state_vectors(SAMPLER, PATH, TEAM, NW, POT);
+    constexpr bool kDense = Chain<TEAM, SAMPLER, POT, PATH, NW>::kDense;
     int used = kVectors;
     ch.off_a = ch.off_b = 0;
-    if constexpr (kVectors == 4) {
+    if constexpr (kVectors - (kDense ? 2 : 0) == 4) {
         ch.off_a = 2 * vec + toff;
         ch.off_b = 3 * vec + toff;
+    }
+    if constexpr (kDense) {  // the last two state vectors (left unset otherwise: setting them changes the other kernels' SASS)
+        ch.off_g = (kVectors - 2) * vec + toff;
+        ch.off_h = (kVectors - 1) * vec + toff;
     }
     {
         double* base = p.scratch_in_smem ? g_smem + (size_t)used * vec + toff
@@ -2638,6 +2719,10 @@ __global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH ==
     ch.for_owned([&](int j) {
         g_smem[ch.off_x + j * ch.kStr] = p.sx[c * p.d + ch.coord(j)];
         g_smem[ch.off_v + j * ch.kStr] = p.sv[c * p.d + ch.coord(j)];
+        if constexpr (kDense) {
+            g_smem[ch.off_g + j * ch.kStr] = p.sg[c * p.d + ch.coord(j)];
+            g_smem[ch.off_h + j * ch.kStr] = p.sh[c * p.d + ch.coord(j)];
+        }
     });
     ch.t = p.st[c];
     ch.horizon = p.shorizon[c];
@@ -2679,6 +2764,10 @@ __global__ void __launch_bounds__(block_threads_rt(TEAM, SAMPLER, PATH), PATH ==
         if (ch.owns(j)) {
             p.sx[c * p.d + ch.coord(j)] = g_smem[ch.off_x + j * ch.kStr];
             p.sv[c * p.d + ch.coord(j)] = g_smem[ch.off_v + j * ch.kStr];
+            if constexpr (kDense) {
+                p.sg[c * p.d + ch.coord(j)] = g_smem[ch.off_g + j * ch.kStr];
+                p.sh[c * p.d + ch.coord(j)] = g_smem[ch.off_h + j * ch.kStr];
+            }
         }
     if (p.accumulate_moments)
         for (int j = 0; j < ch.nown; ++j)

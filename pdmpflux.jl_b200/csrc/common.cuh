@@ -27,17 +27,21 @@ constexpr int kLineShared = 0;       // shared-memory A / B vectors (also every 
 constexpr int kLineTransposed = -1;  // transposed Brent search: every lane keeps the chain's compressed model (chain.cuh)
 constexpr int kLineRegs = 16;        // registers: at most kLineRegs owned coordinates per lane, one team reduction per rate
 
-// shared-memory state vectors of a block before the scratch / flags / moments: x, v and, where the line model keeps
-// them there, A and B
-__host__ __device__ constexpr int state_vectors(int sampler, int path, int team, int line) {
-    return sampler == PDMPFLUX_ZIGZAG && path == kPathFastBrent && team > 1 && line != kLineRegs ? 4 : 2;
+// shared-memory state vectors of a block before the scratch / flags / moments: x, v, where the line model keeps them
+// there A and B, and for the dense Gaussian the maintained g = P (x - mu) and h = P v
+__host__ __device__ constexpr int state_vectors(int sampler, int path, int team, int line, int pot) {
+    return (sampler == PDMPFLUX_ZIGZAG && path == kPathFastBrent && team > 1 && line != kLineRegs ? 4 : 2) +
+           (pot == PDMPFLUX_GAUSS_DENSE ? 2 : 0);
 }
 
 // Thread-per-chain Zig-Zag x Brent is limited by the shared memory its chains' x and v take (16 d bytes per chain):
 // blocks of 64 threads pack the SM with four blocks (8 warps) where blocks of 128 leave room for one or two.
 // The same holds for thread-per-chain BPS / Boomerang / ForwardECMC at d ~ 100 (1.8 kB of state per chain): blocks of
 // one warp.  (Thread-per-chain Zig-Zag with a grid bound is used at small d only and keeps 128.)
-__host__ __device__ constexpr int block_threads_rt(int team, int sampler, int path) {
+// The dense Gaussian keeps four to six d-vectors per chain (64 kB each at d = 2048): its warp-per-chain blocks hold one
+// chain, so that d = 2048 fits and a block's shared memory does not hold the SM to one block of four chains.
+__host__ __device__ constexpr int block_threads_rt(int team, int sampler, int path, int pot) {
+    if (team == 32 && pot == PDMPFLUX_GAUSS_DENSE) return 32;
     if (team != 1) return kBlockThreads;
     if (sampler == PDMPFLUX_ZIGZAG) return path == kPathFastBrent ? 64 : kBlockThreads;
     if (sampler == PDMPFLUX_BPS || sampler == PDMPFLUX_FECMC || sampler == PDMPFLUX_BOOMERANG) return 32;
@@ -50,8 +54,8 @@ constexpr double kEps = 2.220446049250313e-16;
 
 // Device-side potential parameters (owned by pdmpflux_potential_s).
 struct PotParams {
-    const double* vec;   // GAUSS_DIAG: p[d]; LOGREG: X[n*d]
-    const double* vec2;  // LOGREG: y[n]
+    const double* vec;   // GAUSS_DIAG: p[d]; LOGREG: X[n*d]; GAUSS_DENSE: P[d*d] (symmetric)
+    const double* vec2;  // LOGREG: y[n]; GAUSS_DENSE: mu[d]
     double alpha, beta;  // GAUSS_EQUICORR
     double inv_s2;       // LOGREG prior precision
     int64_t n;           // LOGREG rows
@@ -117,6 +121,9 @@ struct KernelParams {
                       // the kernel only writes their non-zero entries
     int vec32;        // X, V, t, horizon, ar are 32-byte aligned: 256-bit (one full sector) stores are legal
     int bulk_rows;    // TEAM > 1: X / V rows go out as TMA bulk copies straight from the shared-memory state
+    // dense Gaussian: g = P (x - mu) and h = P v of every chain (state, in/out), maintained by the kernels
+    double* sg;       // [C][d]
+    double* sh;       // [C][d]
 };
 
 // ---- Blackwell store primitives ---------------------------------------------------------------------------

@@ -279,7 +279,7 @@ int jit_launch(const std::string& source, int sampler_kind, int team, int path, 
     }
     void* args[] = {const_cast<KernelParams*>(&p)};
     const cudaError_t ce = cudaLaunchKernel(reinterpret_cast<const void*>(e->kernel), dim3(grid),
-                                            dim3(block_threads_rt(team, sampler_kind, path)), args, smem, stream);
+                                            dim3(block_threads_rt(team, sampler_kind, path, PDMPFLUX_SOURCE)), args, smem, stream);
     if (ce != cudaSuccess) return pdmpflux_fail_(PDMPFLUX_ERR_CUDA, std::string("skeleton kernel launch (source potential): ") + cudaGetErrorString(ce));
     return PDMPFLUX_OK;
 }

@@ -10,9 +10,10 @@ namespace pdmpflux {
 //   kLineRegs        teams of 8 with at most 16 owned coordinates per lane (d <= 128): register-resident (A_j, B_j),
 //                    team reduction per rate evaluation
 //   kLineShared      the shared-memory A/B arrays (every other team and sampler)
-// launch_for_pot instantiates exactly these; api.cu sizes the shared memory with it.
-inline int brent_line_model(int sampler, int path, int team, int n_own) {
-    if (sampler != PDMPFLUX_ZIGZAG || path != kPathFastBrent || team != 8) return kLineShared;
+// launch_for_pot instantiates exactly these; api.cu sizes the shared memory with it.  The dense Gaussian keeps its g and
+// h next to x and v and uses the shared-memory model only.
+inline int brent_line_model(int sampler, int path, int team, int n_own, int pot) {
+    if (sampler != PDMPFLUX_ZIGZAG || path != kPathFastBrent || team != 8 || pot == PDMPFLUX_GAUSS_DENSE) return kLineShared;
     if (n_own <= 8) return kLineTransposed;
     return n_own <= kLineRegs ? kLineRegs : kLineShared;
 }
@@ -26,10 +27,17 @@ constexpr bool has_fast_path(int sampler, bool affine, int n_special) {
 template <int POT>
 constexpr bool has_fast_path(int sampler) { return has_fast_path(sampler, Pot<POT>::kAffine, Pot<POT>::kSpecial); }
 
+// kernels of the dense Gaussian: the Zig-Zag and BPS fast paths on teams (api.cu: sampler creation admits no other)
+template <int TEAM, int SAMPLER, int PATH>
+constexpr bool dense_built() {
+    return TEAM > 1 && PATH != kPathGeneric && (SAMPLER == PDMPFLUX_ZIGZAG || SAMPLER == PDMPFLUX_BPS);
+}
+
 template <int TEAM, int SAMPLER, int POT, int PATH, int NW = kLineShared>
 cudaError_t launch_one(const KernelParams& p, unsigned grid, size_t smem, cudaStream_t stream) {
     // no fast-path kernel is built where select_path never picks one
-    constexpr bool ok = PATH == kPathGeneric || has_fast_path<POT>(SAMPLER);
+    constexpr bool ok = (PATH == kPathGeneric || has_fast_path<POT>(SAMPLER)) &&
+                        (POT != PDMPFLUX_GAUSS_DENSE || (dense_built<TEAM, SAMPLER, PATH>() && NW == kLineShared));
     if constexpr (!ok) return cudaErrorInvalidValue;
     else {
         auto kern = skeleton_kernel<TEAM, SAMPLER, POT, PATH, NW>;
@@ -37,7 +45,7 @@ cudaError_t launch_one(const KernelParams& p, unsigned grid, size_t smem, cudaSt
             cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
         }
-        kern<<<grid, block_threads_rt(TEAM, SAMPLER, PATH), smem, stream>>>(p);
+        kern<<<grid, block_threads_rt(TEAM, SAMPLER, PATH, POT), smem, stream>>>(p);
         return cudaGetLastError();
     }
 }
@@ -47,7 +55,7 @@ cudaError_t launch_for_pot(int path, const KernelParams& p, unsigned grid, size_
     switch (path) {
     case kPathGeneric: return launch_one<TEAM, SAMPLER, POT, kPathGeneric>(p, grid, smem, stream);
     case kPathFastBrent:
-        if constexpr (TEAM == 8 && SAMPLER == PDMPFLUX_ZIGZAG && Pot<POT>::kAffine) {
+        if constexpr (TEAM == 8 && SAMPLER == PDMPFLUX_ZIGZAG && Pot<POT>::kAffine && POT != PDMPFLUX_GAUSS_DENSE) {
             switch (p.brent_nw) {
             case kLineTransposed: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, kLineTransposed>(p, grid, smem, stream);
             case kLineRegs: return launch_one<TEAM, SAMPLER, POT, kPathFastBrent, kLineRegs>(p, grid, smem, stream);
@@ -68,6 +76,7 @@ cudaError_t launch_for_team(int pot, int path, const KernelParams& p, unsigned g
     case PDMPFLUX_BANANA: return launch_for_pot<TEAM, SAMPLER, PDMPFLUX_BANANA>(path, p, grid, smem, stream);
     case PDMPFLUX_BANANA_README_SCALAR:
         return launch_for_pot<TEAM, SAMPLER, PDMPFLUX_BANANA_README_SCALAR>(path, p, grid, smem, stream);
+    case PDMPFLUX_GAUSS_DENSE: return launch_for_pot<TEAM, SAMPLER, PDMPFLUX_GAUSS_DENSE>(path, p, grid, smem, stream);
     default: return cudaErrorInvalidValue;
     }
 }
@@ -93,6 +102,7 @@ inline LineTraits builtin_line_traits(int pot) {
     case PDMPFLUX_BANANA: return {Pot<PDMPFLUX_BANANA>::kAffine, Pot<PDMPFLUX_BANANA>::kSpecial};
     case PDMPFLUX_BANANA_README_SCALAR:
         return {Pot<PDMPFLUX_BANANA_README_SCALAR>::kAffine, Pot<PDMPFLUX_BANANA_README_SCALAR>::kSpecial};
+    case PDMPFLUX_GAUSS_DENSE: return {Pot<PDMPFLUX_GAUSS_DENSE>::kAffine, Pot<PDMPFLUX_GAUSS_DENSE>::kSpecial};
     default: return {};
     }
 }

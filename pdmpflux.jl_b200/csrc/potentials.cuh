@@ -143,4 +143,24 @@ struct Pot<PDMPFLUX_BANANA_README_SCALAR> {  // every coordinate = x1 + (x2 - (x
     }
 };
 
+// U = (x - mu)' P (x - mu) / 2 with a dense symmetric positive-definite P (pp.vec = P row-major, pp.vec2 = mu).  The
+// gradient needs all of x, not K <= 8 functionals, so the chain keeps g = P (x - mu) and h = P v itself (chain.cuh,
+// kDense) and uses (g_i, h_i) wherever the fast paths take (grad U(x))_i and (H v)_i; the line model is exact.  The
+// members below are never called: they let the generic code that the fast-path kernels compile (but never reach)
+// type-check, and a NaN would show at once if a path did reach them.
+template <>
+struct Pot<PDMPFLUX_GAUSS_DENSE> {
+    static constexpr int K = 0;
+    static constexpr bool kAffine = true;
+    static constexpr int kSpecial = 0;
+    static constexpr bool kSplit = true;
+    __device__ static void accum(const PotParams&, int, double, double*) {}
+    __device__ static double grad(const PotParams&, int, double, const double*) { return CUDART_NAN; }
+    __device__ static void eval(const PotParams&, int, double, double, const double*, const double*, double& g, double& hd) {
+        g = CUDART_NAN; hd = CUDART_NAN;
+    }
+    __device__ static void eval_local(const PotParams&, int, double, double, double& gl, double& hl) { gl = CUDART_NAN; hl = CUDART_NAN; }
+    __device__ static void line_corr(const PotParams&, const double*, const double*, double& ca, double& cb) { ca = 0.0; cb = 0.0; }
+};
+
 }  // namespace pdmpflux

@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _lib
 
-GAUSS_STD, GAUSS_DIAG, GAUSS_EQUICORR, BANANA, BANANA_README_SCALAR, LOGREG, SOURCE = range(7)
+GAUSS_STD, GAUSS_DIAG, GAUSS_EQUICORR, BANANA, BANANA_README_SCALAR, LOGREG, SOURCE, GAUSS_DENSE = range(8)
 
 
 class Potential:
@@ -56,6 +56,26 @@ class GaussEquicorr(Potential):
 
     def params(self, dim):
         return np.array([self.rho])
+
+
+class GaussDense(Potential):
+    """U(x) = (x - mean)' P (x - mean) / 2 with a dense symmetric positive-definite precision matrix P (d <= 2048):
+    a Gaussian with covariance inv(P).  Runs on the fast-path kernels of ZigZag (grid_size=0, or a vectorised grid bound
+    with an exact AD_backend) and BPS (every configuration); other samplers and options raise UnsupportedError when the
+    sampler is built.  The library checks that P is finite, symmetric (to 1e-12 max|P|; it uses (P + P')/2) and positive
+    definite.  RV_diagnostic does not run it."""
+    kind = GAUSS_DENSE
+
+    def __init__(self, precision, mean=None):
+        self.P = np.asarray(precision, dtype=np.float64)
+        if self.P.ndim != 2 or self.P.shape[0] != self.P.shape[1]:
+            raise _lib.ArgumentError(f"GaussDense needs a square precision matrix, got shape {self.P.shape}")
+        self.mean = np.zeros(self.P.shape[0]) if mean is None else np.asarray(mean, dtype=np.float64)
+
+    def params(self, dim):
+        if self.P.shape != (dim, dim) or self.mean.shape != (dim,):
+            raise _lib.DimensionMismatch(f"GaussDense has a {self.P.shape} precision and a {self.mean.shape} mean but dim = {dim}")
+        return np.concatenate([self.P.ravel(), self.mean])
 
 
 class Banana(Potential):
