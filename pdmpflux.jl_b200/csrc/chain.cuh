@@ -75,6 +75,13 @@ __device__ unsigned long long g_phase_clock[kPhases + 1];
 // whose rate changes sign inside the bound's bracket (see Chain::classify_line)
 constexpr int kCrossMax = 12;
 
+// Built-in potentials whose functionals are single coordinates declare kPickFunctionals (potentials.cuh); a potential
+// without the member (source potentials included) is reduced with the butterfly.
+template <class P, class = void>
+struct pick_functionals { static constexpr bool value = false; };
+template <class P>
+struct pick_functionals<P, decltype((void)P::kPickFunctionals)> { static constexpr bool value = P::kPickFunctionals; };
+
 // NW (Zig-Zag + kPathFastBrent only) is the line model of common.cuh.  kLineRegs: compile-time capacity of the
 // owned-coordinate loops; the line model (A_j, B_j) of the owned coordinates then lives in registers (slots >= n_own
 // hold A = B = 0) and the ~40 rate evaluations of a Brent bound touch neither shared memory nor any loop counter.
@@ -296,7 +303,15 @@ struct Chain {
 
     // functionals of the current x and v (one fused multi-value reduction)
     __device__ void compute_functionals() {
-        if constexpr (K > 0) {
+        if constexpr (kTeamSpec && pick_functionals<P>::value) {
+            // L_k = x_k: in the butterfly every lane but the owner adds an exact +0.0 to the owner's 0.0 + x_k, so the
+            // owner's value broadcast plus 0.0 has the same bits (-0.0 included) at 4 shuffles instead of 24
+#pragma unroll
+            for (int k = 0; k < KK; ++k) {
+                Lx[k] = team_bcast<TEAM>(XS(k / TEAM), k % TEAM, mask) + 0.0;
+                Lv[k] = team_bcast<TEAM>(VS(k / TEAM), k % TEAM, mask) + 0.0;
+            }
+        } else if constexpr (K > 0) {
             double acc[2 * KK];
 #pragma unroll
             for (int k = 0; k < 2 * KK; ++k) acc[k] = 0.0;
@@ -1315,13 +1330,15 @@ struct Chain {
     }
 
     __device__ void build_bound_brent(double h) {
-        if constexpr (kCompressed) classify_line(h);
+        if constexpr (kCompressed && !kTeamSpec) classify_line(h);
         Brent s;
         s.lo = 0.0; s.hi = h;
         s.x = __dadd_rn(s.lo, __dmul_rn(kGolden, __dadd_rn(s.hi, -s.lo)));
-        s.fx = -rate_unsigned(s.x);
-        s.stp = 0.0; s.old = 0.0; s.w = s.x; s.v = s.x; s.fw = s.fx; s.fv = s.fx;
-        PDMPFLUX_PHASE(kPhFunc);
+        if constexpr (!kTeamSpec) {
+            s.fx = -rate_unsigned(s.x);
+            s.stp = 0.0; s.old = 0.0; s.w = s.x; s.v = s.x; s.fw = s.fx; s.fv = s.fx;
+            PDMPFLUX_PHASE(kPhFunc);
+        }
         if constexpr (kTeamSpec) {
             // Transposed passes: lane tl of the team takes iterations tl, tl + TEAM, tl + 2 TEAM, ... of the next
             // kSuper * TEAM iterations -- on BASELINE config C2 a whole bound (36 iterations) is one pass.  While golden
@@ -1341,18 +1358,26 @@ struct Chain {
             // So that lane also evaluates the stopping rule of the iteration after it.  When that fires (and the tol
             // step is a new best in the assumed direction) the lane vouches for its iteration and sets the stop bit of
             // the next one: the search ends on the tol step's value without replaying it.
+            // The first pass of a bound also evaluates the starting point: its slots are shifted by one, slot 0 (lane 0,
+            // block 0) holds f(x) of the initial state and slot k + 1 iteration k, so the initial value reaches iteration
+            // 0 through the same rotation as any other and the pass covers the initial point plus 39 iterations.  Later
+            // passes start from a committed state whose f(x) is known and map slot k to iteration k.
             constexpr int S = kSuper;
             auto rot = [&](double v, int j) { return __shfl_sync(mask, v, (tl - j) & (TEAM - 1), TEAM); };
-            bool done = false;
-            for (int it = 0; it < 1000 && !done;) {
+            s.stp = 0.0; s.old = 0.0; s.w = s.x; s.v = s.x;
+            classify_line(h);
+            PDMPFLUX_PHASE(kPhFunc);
+            bool done = false, first_pass = true;
+            for (int it = 0; it < 1000 && !done; first_pass = false) {
+                const int sh = first_pass ? 1 : 0;   // slot of iteration 0
                 const bool right = s.x < (s.hi + s.lo) * 0.5;
                 const double E = right ? s.hi : s.lo;
-                double X[S], W[S], V[S];
+                double X[S], W[S], V[S];   // the state at the start of the iteration of slot TEAM b + tl
                 {
                     double mx = s.x, mw = s.w, mv = s.v;
 #pragma unroll
                     for (int k = 0; k < TEAM - 1; ++k) {
-                        if (k < tl) {
+                        if (k < tl - sh) {
                             const double u = __dadd_rn(mx, __dmul_rn(kGolden, E - mx));
                             mv = mw; mw = mx; mx = u;
                         }
@@ -1363,8 +1388,10 @@ struct Chain {
                     for (int b = 1; b < S; ++b) {
 #pragma unroll
                         for (int k = 0; k < TEAM; ++k) {
-                            const double u = __dadd_rn(mx, __dmul_rn(kGolden, E - mx));
-                            mv = mw; mw = mx; mx = u;
+                            if (b > 1 || k > 0 || tl >= sh) {   // slot TEAM of the first pass is iteration TEAM - 1
+                                const double u = __dadd_rn(mx, __dmul_rn(kGolden, E - mx));
+                                mv = mw; mw = mx; mx = u;
+                            }
                         }
                         X[b] = mx; W[b] = mw; V[b] = mv;
                     }
@@ -1374,12 +1401,14 @@ struct Chain {
                 bool asok[S], tolok[S];
 #pragma unroll
                 for (int b = 0; b < S; ++b) {
-                    const bool first = (b == 0) && (tl == 0);
+                    const bool first = (b == 0) && (tl == sh);
+                    const bool start = (b == 0) && (tl < sh);   // slot 0 of the first pass: the initial point
                     const double moving = first ? (right ? s.lo : s.hi) : W[b];
                     const double lo_ = right ? moving : s.lo, hi_ = right ? s.hi : moving;
                     double mid, og, gstp;
                     U[b] = brent_golden(lo_, hi_, X[b], TOL[b], mid, og, gstp);
-                    const bool stop = fabs(X[b] - mid) <= fma(hi_ - lo_, -0.5, TOL[b] + TOL[b]);
+                    if (start) U[b] = s.x;
+                    const bool stop = !start & (fabs(X[b] - mid) <= fma(hi_ - lo_, -0.5, TOL[b] + TOL[b]));
                     const bool dir = (X[b] < mid) == right;
                     asok[b] = dir & (fabs(gstp) >= TOL[b]);
                     // tol step: the stopping rule of the next iteration, from the state this one leaves when it is a
@@ -1388,7 +1417,7 @@ struct Chain {
                     double tol2, mid2, og2, gstp2;
                     brent_golden(lo2, hi2, U[b], tol2, mid2, og2, gstp2);
                     const bool stop2 = fabs(U[b] - mid2) <= fma(hi2 - lo2, -0.5, tol2 + tol2);
-                    tolok[b] = dir & (fabs(gstp) < TOL[b]) & ((U[b] < X[b]) != right) & stop2 &
+                    tolok[b] = !start & dir & (fabs(gstp) < TOL[b]) & ((U[b] < X[b]) != right) & stop2 &
                                (b < S - 1 || tl < TEAM - 1);
                     stopmask |= (unsigned long long)(stop ? 1u : 0u) << (TEAM * b + tl);   // my bits; merged below
                 }
@@ -1402,7 +1431,11 @@ struct Chain {
                     for (int b = 0; b < S; ++b) {
                         const double r1 = rot(F[b], 1), r2 = rot(F[b], 2), r3 = rot(F[b], 3);
                         Brent m;
-                        if (b == 0) {
+                        if (b == 0 && first_pass) {   // f(x) = fw = fv of the initial state come from slot 0
+                            m.fx = r1;
+                            m.fw = tl >= 2 ? r2 : r1;
+                            m.fv = tl >= 3 ? r3 : (tl == 2 ? r2 : r1);
+                        } else if (b == 0) {
                             m.fx = tl >= 1 ? r1 : s.fx;
                             m.fw = tl >= 2 ? r2 : (tl == 1 ? s.fx : s.fw);
                             m.fv = tl >= 3 ? r3 : (tl == 2 ? s.fx : (tl == 1 ? s.fw : s.fv));
@@ -1412,7 +1445,8 @@ struct Chain {
                             m.fv = tl >= 3 ? r3 : r3p;
                         }
                         r1p = r1; r2p = r2; r3p = r3;
-                        const bool first = (b == 0) && (tl == 0);
+                        const bool first = (b == 0) && (tl == sh);
+                        const bool start = (b == 0) && (tl < sh);
                         const double moving = first ? (right ? s.lo : s.hi) : W[b];
                         m.lo = right ? moving : s.lo;
                         m.hi = right ? s.hi : moving;
@@ -1422,17 +1456,17 @@ struct Chain {
                         const bool para = brent_parabola(m, TOL[b], pp, qq);
                         const bool best = !para & (F[b] < m.fx);
                         const bool fin = best & tolok[b];   // a tol step after which the search stops
-                        goodmask |= (unsigned long long)(((best & asok[b]) | fin) ? 1u : 0u) << (TEAM * b + tl);
+                        goodmask |= (unsigned long long)(((best & asok[b]) | fin | start) ? 1u : 0u) << (TEAM * b + tl);
                         stopmask |= (unsigned long long)(fin ? 1u : 0u) << (TEAM * b + tl + 1);
                     }
                 }
                 stopmask = team_or64<TEAM>(stopmask, mask);
                 goodmask = team_or64<TEAM>(goodmask, mask);
                 constexpr int N = S * TEAM;
-                const int nterm = stopmask ? __ffsll((long long)stopmask) - 1 : N;   // first iteration that stops
-                const int nbad = __ffsll((long long)~goodmask) - 1;                   // first iteration not as assumed (>= N: none)
-                const int nc = min(nterm, min(nbad, N));                              // iterations 0 .. nc-1 stand
-                // value a lane noted for iteration `step` (team-uniform argument)
+                const int nterm = stopmask ? __ffsll((long long)stopmask) - 1 : N;   // first slot whose iteration stops
+                const int nbad = __ffsll((long long)~goodmask) - 1;                   // first slot not as assumed (>= N: none)
+                const int nc = min(nterm, min(nbad, N));                              // slots 0 .. nc-1 stand
+                // value a lane noted for slot `step` (team-uniform argument)
                 auto at = [&](const double (&arr)[S], int step) {
                     const int bb = step / TEAM;
                     double sel = arr[0];
@@ -1440,13 +1474,14 @@ struct Chain {
                     for (int b = 1; b < S; ++b) sel = (bb == b) ? arr[b] : sel;
                     return team_bcast<TEAM>(sel, step & (TEAM - 1), mask);
                 };
-                it += nc;
+                it += nc - sh;
                 PDMPFLUX_PHASE(kPhPass);
                 if (nterm <= nbad && nterm < N) {   // the stopping rule fired: only the best value is needed
                     if (nterm >= 1) s.fx = at(F, nterm - 1);
                     done = true;
                 } else {
-                    if (nc >= 1) {                  // the state at the start of iteration nc
+                    if (first_pass) s.fx = s.fw = s.fv = team_bcast<TEAM>(F[0], 0, mask);
+                    if (nc > sh) {                  // the state at the start of the iteration of slot nc
                         const double xn = (nc < N) ? at(X, min(nc, N - 1)) : team_bcast<TEAM>(ulast, TEAM - 1, mask);
                         const double wn = at(X, nc - 1);
                         const double vn = nc >= 2 ? at(X, nc - 2) : s.w;

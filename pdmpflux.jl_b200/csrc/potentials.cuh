@@ -99,6 +99,7 @@ struct Pot<PDMPFLUX_BANANA> {  // L0 = x_1, L1 = x_2 (1-based); r = x2 - x1^2 + 
     static constexpr int K = 2;
     static constexpr bool kAffine = true;   // coordinates >= 2 are standard-Gaussian
     static constexpr int kSpecial = 2;      // coordinates 0, 1 are polynomial in t and functions of (L0, L1) only
+    static constexpr bool kPickFunctionals = true;   // L_k = x_k for k < K: picks, not sums (chain.cuh: compute_functionals)
     __device__ static void accum(const PotParams&, int i, double xi, double* acc) {
         if (i == 0) acc[0] += xi;
         if (i == 1) acc[1] += xi;

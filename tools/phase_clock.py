@@ -4,8 +4,8 @@ Builds a separate copy of the library with -DPDMPFLUX_PHASE_CLOCK into OUT/ (the
 the bench workload (Zig-Zag, banana d = 50, Brent bounds, Philox draws, 4096 chains x 1000 events) on it once to warm
 up and once counted, and prints the lane cycles per event in each phase:
 
-  func    compute_functionals, line model, classification, the first rate of the Brent search
-  pass    speculative passes of the transposed Brent search
+  func    compute_functionals, line model, classification
+  pass    speculative passes of the transposed Brent search (the first one also evaluates the bound's starting point)
   replay  commit of a pass and the one-at-a-time iterations after it (or the broadcast of the final value)
   next    next_event and its exponential draw (after a bound and after a rejection)
   rate    the rate at the proposal and the accept uniform
